@@ -2,6 +2,7 @@
 """bench.py — throughput of the CAV-Gym stepping hot path on B200 (driver contract in the task prompt).
 
     python bench.py --gpus 1 --steps 1000 --warmup 100             # our arm
+    python bench.py --gpus 1 --steps 1000 --warmup 100 --dump-outputs DIR   # also write the last timed step's results
     python bench.py --impl reference --gpus 1 --steps 200 --warmup 10   # CPU arm (oracle port, all host threads)
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
@@ -29,7 +30,6 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 N_ENVS = 65536          # per GPU (weak scaling)
 SEGMENT = 250           # steps replayed from a fresh reset before the whole batch is reset again: a finished env stays frozen
                         # (and uncounted) until then — 3 % of the env-steps at 250, 10 % at 500 (the ego finishes at step 901)
-REGION_REPEATS = 50     # the --steps-long timed region is repeated this many times back to back (all launches pre-enqueued)
 CHUNK = 250             # steps fused per cavgym_replay launch (50: 16.0, 100: 17.9, 250: 20.3, 500: 20.8 G env-steps/s)
 HBM_ENVS = 4 * 1024 * 1024
 HBM_ADVANCE = 300        # unrecorded steps before the HBM-config trace: envs are mid-episode, pedestrians mid-crossing
@@ -135,6 +135,18 @@ def make_trace(torch, device, n_envs, n_steps, dtype, env_offset, advance=0):
     return init, actions
 
 
+def dump_outputs(directory, arrays):
+    """Write what the last timed step returned to its caller (cavgym_replay: state [M, 4, N], reward [M, N], done, winner,
+    tangent [N]) as DIR/<name>.npy, so that two builds can be compared output for output: the trace and the initial state
+    are generated from fixed seeds, so the same arguments replay the same inputs.  Real arrays keep the run's dtype;
+    done / winner / tangent are stored as float64 (exact).  About 7 MB at float64."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, tensor in arrays.items():
+        data = tensor.cpu().numpy()
+        np.save(os.path.join(directory, f"{name}.npy"), data if data.dtype.kind == "f" else data.astype(np.float64))
+
+
 def run_ours(args):
     chunk = max(1, min(int(args.chunk), SEGMENT, args.steps))   # steps fused per cavgym_replay launch
     segment = SEGMENT // chunk * chunk                          # whole launches between resets (240 steps at 20 per launch)
@@ -171,7 +183,7 @@ def run_ours(args):
     def ptr(t):
         return C.c_void_p(t.data_ptr())
 
-    launch_events, region_events, launch_no = [], [], [0]
+    launch_events, launch_no, last_step = [], [0], [0]
 
     def advance(n_steps, cursor, timed):
         """Replay n_steps starting at trace position `cursor` (resetting every `segment` steps); returns new cursor."""
@@ -185,6 +197,7 @@ def run_ours(args):
                 a.record()
             at = (launch_no[0] % slots) * chunk
             launch_no[0] += 1
+            last_step[0] = at + take - 1          # slab row of the results of the last step replayed so far
             check(lib.cavgym_replay(handle, take, ptr(actions[cursor]), ptr(slab["state"][at]), ptr(slab["reward"][at]),
                                     ptr(slab["done"][at]), ptr(slab["winner"][at]), ptr(slab["tangent"][at]), stream))
             if timed:
@@ -201,38 +214,33 @@ def run_ours(args):
         torch.cuda.synchronize(device)
 
     # ---- device-resident throughput (value) -------------------------------------------------
-    # The timed region is `--steps` steps (resets included), repeated REGION_REPEATS times back to back.  Every launch of
-    # every repetition is enqueued while a gate kernel keeps the stream busy, so no host launch latency sits between
-    # the events: they time the GPU, not the Python loop (at --steps 20 one region is a single ~70 us launch).
+    # The timed region is `--steps` steps (resets included).  All its launches are enqueued while a gate kernel keeps the
+    # stream busy, so no host launch latency sits between the events: they time the GPU, not the Python loop.
     advance(args.warmup, 0, False)
-    cursor = 0   # the first timed region starts from a fresh reset: regions tile the segment-step trace whenever --steps divides it
+    cursor = 0   # pass A starts from a fresh reset, pass B where pass A ended
     barrier()
-    before, launches_before = env.stats(), env.launch_count()
     sampler = ClockSampler(local)
     sampler.start()
     sampler.ready.wait(timeout=10)    # NVML initialised before the timed region starts
-    repeats = max(1, args.repeats)
     launches_per_region = -(-args.steps // chunk) + args.steps // segment + 2
     barrier()
     if args.profile_region:      # ncu --profile-from-start off: capture exactly the timed region
         torch.cuda.profiler.start()
-    torch.cuda._sleep(int((4e-3 + 4e-5 * repeats * launches_per_region) * 1.9e9))
-    # Pass A (per-launch statistics): a CUDA event before and after every launch.  An event between two launches also
-    # serialises them, so this pass shows each launch in isolation (no programmatic dependent launch overlap).
-    for _ in range(repeats):   # a region starts at its first launch's start event and ends at its last launch's stop event
-        first = len(launch_events)
-        cursor = advance(args.steps, cursor, True)
-        region_events.append((launch_events[first][0], launch_events[-1][1]))
-    queued_ahead = not region_events[0][0].query()   # the GPU had not reached the first event when the host finished enqueuing
+    torch.cuda._sleep(int((4e-3 + 4e-5 * launches_per_region) * 1.9e9))
+    # Pass A (per-launch statistics, untimed for `value`): a CUDA event before and after every launch.  An event between two
+    # launches also serialises them, so this pass shows each launch in isolation (no programmatic dependent launch overlap).
+    cursor = advance(args.steps, cursor, True)
+    queued_ahead = not launch_events[0][0].query()   # the GPU had not reached the first event when the host finished enqueuing
     barrier()
+    region_ms = launch_events[0][0].elapsed_time(launch_events[-1][1])
     mid, launches_mid = env.stats(), env.launch_count()
-    # Pass B (the measurement): the same launches back to back as a caller issues them — nothing between them — with ONE
-    # event pair around all repetitions: consecutive replay launches overlap head and tail (launch_replay_tma).
-    torch.cuda._sleep(int((4e-3 + 4e-5 * repeats * launches_per_region) * 1.9e9))
+    # Pass B (the measurement): the next `--steps` steps of the trace, launched back to back as a caller issues them —
+    # nothing between them — with ONE event pair around them: consecutive replay launches overlap head and tail
+    # (launch_replay_tma).
+    torch.cuda._sleep(int((4e-3 + 4e-5 * launches_per_region) * 1.9e9))
     start_b, stop_b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     start_b.record()
-    for _ in range(repeats):
-        cursor = advance(args.steps, cursor, False)
+    advance(args.steps, cursor, False)
     stop_b.record()
     queued_ahead = queued_ahead and not start_b.query()
     barrier()
@@ -240,9 +248,10 @@ def run_ours(args):
         torch.cuda.profiler.stop()
     clocks = sampler.stop()
     elapsed_ms = start_b.elapsed_time(stop_b)
-    region_ms = sorted(a.elapsed_time(b) for a, b in region_events)
     after, launches_after = env.stats(), env.launch_count()
     live_env_steps = after["env_steps"] - mid["env_steps"]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {name: slab[name][last_step[0]] for name in slab})
     # stats() itself launches one reduction kernel per call: not part of the timed region
     gpu_launches = launches_after - launches_mid - 1
     isolated_ms = sum(a.elapsed_time(b) for a, b, _ in launch_events) / len(launch_events)
@@ -255,7 +264,7 @@ def run_ours(args):
     value = total_env_steps / (elapsed_ms * 1e-3)
 
     # roofline of the dominant kernel: algorithmic bytes per launch / mean launch duration (CUDA events around each launch)
-    live_fraction = live_env_steps / float(n * args.steps * repeats)
+    live_fraction = live_env_steps / float(n * args.steps)
     bytes_per_launch = bytes_env_step * n * steps_per_launch * live_fraction
     achieved = bytes_per_launch / (kernel_ms / replay_launches * 1e-3) / 1e9
     kernel_name = f"replay_tma_kernel<{'double' if dtype == 'float64' else 'float'},2,false>"
@@ -279,21 +288,18 @@ def run_ours(args):
                 "note": "65,536 envs: the state (4 MiB) stays in registers for the whole launch; actions stream in and "
                         "trajectories stream out through HBM (slabs larger than L2)"}
 
-    median_region = region_ms[len(region_ms) // 2]
     out = {"metric": "env_steps_per_sec", "value": value, "unit": "env-steps/s", "n_gpus": world, "steps": args.steps,
-           "warmup": args.warmup, "ms_per_step": elapsed_ms / (args.steps * repeats), "higher_is_better": True, "scaling": "weak",
+           "warmup": args.warmup, "ms_per_step": elapsed_ms / args.steps, "higher_is_better": True, "scaling": "weak",
            "vs_baseline": None, "dtype": "f64" if dtype == "float64" else "f32", "data": "synthetic",
            "body_steps_per_sec": value * m,
-           "timed_region": {"steps": args.steps, "repeats": repeats, "total_ms": elapsed_ms,
-                            "region_ms_median": median_region, "region_ms_min": region_ms[0], "region_ms_max": region_ms[-1],
-                            "value_at_median_region": world * live_env_steps / repeats / (median_region * 1e-3),
+           "timed_region": {"steps": args.steps, "total_ms": elapsed_ms, "region_ms_per_launch_events": region_ms,
                             "launches_queued_before_first_event": bool(queued_ahead),
-                            "note": "value = live env-steps of all repeats / device time between ONE event pair around all repeats, launches "
-                                    "issued back to back behind a gate kernel (max over ranks); region_ms_* are from a separate pass with an "
-                                    "event pair around every region (which serialises consecutive launches)"},
+                            "note": "value = live env-steps / device time between ONE event pair around the --steps steps, launches "
+                                    "issued back to back behind a gate kernel (max over ranks); region_ms_per_launch_events is from a "
+                                    "separate pass over as many steps with an event pair around every launch (which serialises them)"},
            "config": {"workload": "C2: pedestrians scenario (Car + SpawnPedestrian) x 65,536 envs per GPU, replayed joint "
                                   f"actions (on-device RandomConstrained eps=0.01 trace), cavgym_replay {steps_per_launch:g} steps/launch, "
-                                  f"trajectories recorded, region of {args.steps} steps repeated {repeats}x",
+                                  f"trajectories recorded, {args.steps} timed steps",
                       "envs_per_gpu": n, "bodies": m, "segment": segment,
                       "l2": f"{slots} rotating trajectory slabs ({slab_steps * 5.24e6 / 1e9:.2f} GB) and the action trace (1 GB) exceed L2; state is register resident",
                       "live_fraction": round(live_fraction, 4)},
@@ -720,11 +726,11 @@ def main():
     parser.add_argument("--e2e-steps", type=int, default=200)
     parser.add_argument("--cpu-seconds", type=float, default=15.0)
     parser.add_argument("--chunk", type=int, default=CHUNK, help="steps fused per cavgym_replay launch (at most --steps)")
-    parser.add_argument("--repeats", type=int, default=REGION_REPEATS, help="back-to-back repetitions of the --steps-long timed region")
     parser.add_argument("--skip-hbm", action="store_true")
     parser.add_argument("--skip-cpu", action="store_true")
     parser.add_argument("--skip-configs", action="store_true", help="skip the C3 / C4 / C5 side measurements")
     parser.add_argument("--profile-region", action="store_true", help="cudaProfilerStart/Stop around the timed region (ncu --profile-from-start off)")
+    parser.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step (rank 0's envs) as DIR/<name>.npy")
     args = parser.parse_args()
     if args.warmup < 3:
         args.warmup = 3

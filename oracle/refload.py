@@ -1,10 +1,10 @@
 """Import the CAV-Gym reference VERBATIM from /root/reference with stand-ins for
 its un-vendored dependencies.  TEST INFRASTRUCTURE ONLY — build container only.
 
-/root/reference does not exist on the GPU box, so nothing under tests/ (gpu or
-not), bench.py or __graft_entry__.smoke() may import this module at run time;
-it is used by oracle/gen_golden.py to produce the fixtures in tests/golden/ and
-by the optional `reference`-marked tests that skip when the tree is absent.
+The reference is not part of this repository, so nothing under tests/ (gpu or
+not), bench.py or __graft_entry__.smoke() may call load(): it is used by
+oracle/gen_*golden.py to produce the fixtures in tests/golden/, which the
+tests compare with.
 
 Stand-ins (oracle/standins/): gym 0.17.2 subset, shapely.geometry subset (exact
 convex predicates), enforce_typing (identity), and `np.float = float` because

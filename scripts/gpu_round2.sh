@@ -21,7 +21,7 @@ if has bench; then
   timeout 900 python bench.py --steps 20 --warmup 5 > $out/${tag}_bench.json 2> $out/${tag}_bench.err; echo "bench rc=$?"
   tail -3 $out/${tag}_bench.err
   timeout 600 python bench.py --impl reference --steps 20 --warmup 5 > $out/${tag}_bench_ref.json 2> $out/${tag}_bench_ref.err; echo "ref rc=$?"
-  timeout 900 python bench.py --steps 1000 --warmup 100 --repeats 4 --skip-configs --skip-cpu --skip-hbm > $out/${tag}_bench_1000.json 2> $out/${tag}_bench_1000.err; echo "bench1000 rc=$?"
+  timeout 900 python bench.py --steps 4000 --warmup 100 --skip-configs --skip-cpu --skip-hbm > $out/${tag}_bench_1000.json 2> $out/${tag}_bench_1000.err; echo "bench1000 rc=$?"
   kill $smi
 fi
 if has list; then   # launch list of the bench command's TIMED REGION (cudaProfilerStart/Stop around it; same command line otherwise)

@@ -1,8 +1,6 @@
 import os
 import sys
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
@@ -10,12 +8,3 @@ if ROOT not in sys.path:
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    from oracle import refload
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
-    for item in items:
-        if "reference" in item.keywords and not refload.available():
-            item.add_marker(skip_ref)

@@ -8,7 +8,8 @@ import numpy as np
 from cavgym_b200.scenario import AgentSpec, compile_scenario
 
 GOLDEN_DIR = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-GOLDEN_CASES = sorted(f[:-4] for f in os.listdir(GOLDEN_DIR) if f.endswith(".npz") and f != "geometry_kat.npz" and not f.startswith(("info_", "learn_")))
+GOLDEN_CASES = sorted(f[:-4] for f in os.listdir(GOLDEN_DIR)
+                      if f.endswith(".npz") and f not in ("geometry_kat.npz", "scenario_tables.npz") and not f.startswith(("info_", "learn_")))
 LEARN_CASES = sorted(f[:-4] for f in os.listdir(GOLDEN_DIR) if f.startswith("learn_") and f.endswith(".npz"))   # oracle/gen_learning_golden.py
 
 
@@ -29,6 +30,12 @@ def load_info_golden(name):
     """(meta, state [T, M, 4], body_polygons [T, M, 8], road_angles [T, M]) recorded from the reference's env.info()."""
     data = np.load(os.path.join(GOLDEN_DIR, f"{name}.npz"))
     return json.loads(bytes(data["meta"]).decode()), data["state"], data["body_polygons"], data["road_angles"]
+
+
+def load_scenario_tables(name):
+    """CompiledScenario.tables() recorded for the reference's objects of one stock scenario (oracle/gen_tables_golden.py)."""
+    data = np.load(os.path.join(GOLDEN_DIR, "scenario_tables.npz"))
+    return {part: data[f"{name}/{part}"].tobytes() for part in ("header", "bodies", "spawns")}
 
 
 def env_config_from(cfg):

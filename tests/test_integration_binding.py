@@ -1,5 +1,5 @@
 """integration/batched.py — the binding INTEGRATION.md §A tells a CAV-Gym maintainer to add — run for real: against the
-unmodified reference's objects on CPU (tables only), and on the GPU against a reference trace."""
+tables recorded for the unmodified reference's objects on CPU, and on the GPU against a reference trace."""
 import copy
 import importlib.util
 import os
@@ -19,19 +19,20 @@ def binding():
     return module
 
 
-@pytest.mark.reference
 def test_binding_builds_its_tables_from_the_reference_env():
+    """The walk integration/batched.py makes over an env (bodies, constants, env_config, time_resolution) gives the tables
+    recorded for the reference's own pelican-crossing env (tests/golden/scenario_tables.npz, oracle/gen_tables_golden.py)."""
     from oracle import refload
+    from cavgym_b200.config import make_config
     from cavgym_b200.scenario import AgentSpec, compile_scenario
-    mods = refload.load()
+    from helpers import load_scenario_tables
     data = refload.stock_config_dict(scenario="pelican-crossing", tester="random", seed=3, collisions="all")
-    config = mods["config"].make_config(copy.deepcopy(data))
-    _, env, _, _ = config.setup()
-    assert type(env).__module__.startswith("examples.environments")            # the reference's env object
+    _, env, _, _ = make_config(copy.deepcopy(data)).setup()
     tables = compile_scenario(env.bodies, env.constants, env.env_config, [AgentSpec("external") for _ in env.bodies],
                               time_resolution=env.time_resolution).tables()
     assert len(tables["bodies"]) > 0 and tables["header"][:4] == (5).to_bytes(4, "little")
-    assert binding().BatchedCAVEnv.step.__doc__      # the module imports with the reference tree on sys.path
+    assert tables == load_scenario_tables("binding_pelican-crossing")
+    assert binding().BatchedCAVEnv.step.__doc__      # the module imports
 
 
 @pytest.mark.gpu
