@@ -2,6 +2,7 @@
 
 Public entry points:
   BatchedCAVEnv          tensor API over N environments (engine.py)
+  EnvSnapshot            saved per-env state of some of its environments (BatchedCAVEnv.save_envs)
   library.environment.CAVEnv   single-environment compat view (reference protocol)
   make / register        env-id registry ('Pedestrians-v0', ... as the reference's examples/__init__.py)
   Config / make_config   config.json scenarios (config.py)
@@ -11,9 +12,9 @@ __version__ = "0.1.0"
 
 
 def __getattr__(name):
-    if name == "BatchedCAVEnv":
-        from .engine import BatchedCAVEnv
-        return BatchedCAVEnv
+    if name in ("BatchedCAVEnv", "EnvSnapshot"):
+        from . import engine
+        return getattr(engine, name)
     if name in ("make", "register"):
         from . import examples
         return getattr(examples, name)

@@ -51,6 +51,21 @@ class CavEpisodeRow(C.Structure):
                 ("liveness_sum", C.c_int32)]
 
 
+CAV_SNAPSHOT_VERSION = 1
+
+
+class CavSnapshotLayout(C.Structure):
+    _fields_ = [("version", C.c_int32), ("dtype", C.c_int32), ("m", C.c_int32), ("reserved", C.c_int32), ("k", C.c_int64),
+                ("real_rows", C.c_int64), ("i32_rows", C.c_int64), ("u8_rows", C.c_int64), ("real_offset", C.c_int64),
+                ("i32_offset", C.c_int64), ("u8_offset", C.c_int64), ("total_bytes", C.c_int64), ("fingerprint", C.c_uint64)]
+
+
+class CavEngineState(C.Structure):
+    _fields_ = [("version", C.c_int32), ("dtype", C.c_int32), ("m", C.c_int32), ("reserved", C.c_int32), ("n", C.c_int64),
+                ("shard", C.c_int64), ("t_global", C.c_int64), ("seed", C.c_uint64), ("fingerprint", C.c_uint64),
+                ("tau", C.c_double), ("counters", C.c_int64 * CAV_N_STATS)]
+
+
 class CavScenario(C.Structure):
     _fields_ = [("n_bodies", C.c_int32), ("n_types", C.c_int32), ("n_roads", C.c_int32), ("n_statics", C.c_int32),
                 ("n_spawns", C.c_int32), ("terminate_collisions", C.c_int32), ("terminate_ego_zones", C.c_int32),
@@ -79,6 +94,12 @@ PROTOTYPES = {
     "cavgym_step_host_f32": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cavgym_reset_host": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cavgym_info": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, c_stream]),
+    "cavgym_snapshot_layout": (C.c_int, [c_engine_p, C.c_int64, C.POINTER(CavSnapshotLayout)]),
+    "cavgym_save_envs": (C.c_int, [c_engine_p, C.c_void_p, C.c_int64, C.c_void_p, c_stream]),
+    "cavgym_load_envs": (C.c_int, [c_engine_p, C.c_void_p, C.c_int64, C.c_void_p, c_stream]),
+    "cavgym_fork_envs": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_int64, c_stream]),
+    "cavgym_save_engine": (C.c_int, [c_engine_p, C.POINTER(CavEngineState)]),
+    "cavgym_load_engine": (C.c_int, [c_engine_p, C.POINTER(CavEngineState)]),
     "cavgym_stats": (C.c_int, [c_engine_p, C.POINTER(C.c_int64)]),
     "cavgym_set_episode_log": (C.c_int, [c_engine_p, C.c_int64]),
     "cavgym_drain_episodes": (C.c_int, [c_engine_p, C.c_void_p, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),

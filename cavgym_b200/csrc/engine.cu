@@ -2,10 +2,12 @@
 // conversion, kernel dispatch, the pipelined host-buffer step, statistics and the
 // stand-alone per-function kernels.  No torch types; callers pass raw device pointers.
 #include <cmath>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 #ifndef CAV_HOST_CTAS_PER_SM
@@ -19,6 +21,7 @@
 #endif
 #include "kernels_team.cuh"
 #include "kernels_tma.cuh"   // (tma_span, kReplayTile for the replay launch chain; includes kernels_small.cuh)
+#include "kernels_snapshot.cuh"
 
 namespace cav {
 
@@ -448,6 +451,9 @@ struct CavEngine {
   int32_t* d_winner = nullptr;
   unsigned long long* d_scratch = nullptr;
   void* d_quads = nullptr;  // Quad<R>[CAV_MAX_ROADS + CAV_MAX_STATICS] in the engine's type: corner lists for the general fallbacks
+  uint64_t fingerprint = 0;      // of the scenario tables' contents (scenario_fingerprint)
+  void* d_stage = nullptr;       // cavgym_fork_envs: snapshot of the sources, grown on demand, freed by cavgym_destroy
+  size_t stage_bytes = 0;
 
   size_t real_size() const { return dtype == CAV_F64 ? 8 : 4; }
 };
@@ -596,6 +602,103 @@ static int replay_typed(CavEngine* eng, const DevScenario<R>& sc, EnvBuffers<R> 
   return CAV_OK;
 }
 
+// ---------------------------------------------------------------- snapshots (kernels_snapshot.cuh)
+// 64-bit FNV-1a over the scenario's contents: the CavScenario header up to its two pointers, then the spawn and body rows.
+// None of the three structs has padding, so equal tables give equal bytes wherever they were compiled.
+static uint64_t scenario_fingerprint(const CavScenario& sc) {
+  uint64_t h = 0xcbf29ce484222325ull;
+  auto mix = [&h](const void* p, size_t bytes) {
+    const unsigned char* c = static_cast<const unsigned char*>(p);
+    for (size_t i = 0; i < bytes; ++i) { h ^= c[i]; h *= 0x100000001b3ull; }
+  };
+  mix(&sc, offsetof(CavScenario, spawns));
+  if (sc.n_spawns > 0) mix(sc.spawns, sizeof(CavSpawn) * (size_t)sc.n_spawns);
+  mix(sc.bodies, sizeof(CavBody) * (size_t)sc.n_bodies);
+  return h;
+}
+
+static void snapshot_layout(const CavEngine* eng, int64_t k, CavSnapshotLayout* out) {
+  auto align = [](int64_t bytes) { return (bytes + 255) & ~(int64_t)255; };
+  std::memset(out, 0, sizeof(*out));
+  out->version = CAV_SNAPSHOT_VERSION;
+  out->dtype = eng->dtype;
+  out->m = eng->m;
+  out->k = k;
+  out->real_rows = (int64_t)eng->m * (4 + 2 + CAV_AGENT_WORDS + 2);   // state, action, agent, cs
+  out->i32_rows = (int64_t)eng->m + 4;                                 // liveness, t_ep, episode, winner, active
+  out->u8_rows = 2;                                                    // done, err
+  out->real_offset = 0;
+  out->i32_offset = align(out->real_rows * k * (int64_t)eng->real_size());
+  out->u8_offset = out->i32_offset + align(out->i32_rows * k * 4);
+  out->total_bytes = out->u8_offset + align(out->u8_rows * k);
+  out->fingerprint = eng->fingerprint;
+}
+
+template <typename T>
+static void add_rows(SnapTable<T>& t, void* engine, char* snap, int64_t rows) {
+  const int s = t.n_seg++;
+  t.eng[s] = static_cast<T*>(engine);
+  t.snap[s] = reinterpret_cast<T*>(snap);
+  t.row_end[s] = (s ? t.row_end[s - 1] : 0) + rows;
+}
+
+// Every row of the k selected envs between the engine and `snap` (laid out by snapshot_layout): 3 launches in fp64 (8-, 4-
+// and 1-byte rows), 2 in fp32 (the 4-byte reals share a launch with the int32 rows).
+template <typename R>
+static int move_envs(CavEngine* eng, const EnvBuffers<R>& buf, const int64_t* idx, int64_t k, char* snap, bool to_snapshot,
+                     cudaStream_t stream) {
+  using W = typename std::conditional<sizeof(R) == 8, unsigned long long, uint32_t>::type;
+  CavSnapshotLayout L;
+  snapshot_layout(eng, k, &L);
+  const int64_t m = eng->m;
+  SnapTable<W> reals{};
+  SnapTable<uint32_t> words{};
+  SnapTable<uint8_t> bytes{};
+  char* p = snap + L.real_offset;
+  const int64_t real_row = k * (int64_t)sizeof(R);
+  add_rows(reals, buf.state, p, m * 4);                  p += m * 4 * real_row;
+  add_rows(reals, buf.action, p, m * 2);                 p += m * 2 * real_row;
+  add_rows(reals, buf.agent, p, m * CAV_AGENT_WORDS);    p += m * CAV_AGENT_WORDS * real_row;
+  add_rows(reals, buf.cs, p, m * 2);
+  auto add_ints = [&](SnapTable<uint32_t>& ints) {
+    char* q = snap + L.i32_offset;
+    add_rows(ints, buf.liveness, q, m);                  q += m * k * 4;
+    add_rows(ints, buf.t_ep, q, 1);                      q += k * 4;
+    add_rows(ints, buf.episode, q, 1);                   q += k * 4;
+    add_rows(ints, buf.winner, q, 1);                    q += k * 4;
+    add_rows(ints, buf.active, q, 1);
+  };
+  if constexpr (sizeof(R) == 4) add_ints(reals);   // fp32: the int32 rows continue the 4-byte table
+  else add_ints(words);
+  add_rows(bytes, buf.done, snap + L.u8_offset, 1);
+  add_rows(bytes, buf.err, snap + L.u8_offset + k, 1);
+  const char* what = to_snapshot ? "snapshot gather kernel" : "snapshot scatter kernel";
+  if (!idx && k % 16 == 0) {
+    SnapTable<uint4> wide{};
+    append_wide(wide, reals);
+    append_wide(wide, words);
+    append_wide(wide, bytes);
+    wide.n = wide.k = k / 16;
+    wide.idx = nullptr;
+    wide.to_snapshot = to_snapshot ? 1 : 0;
+    launch_snapshot(wide, stream);
+    return launch_check(eng, what);
+  }
+  auto run = [&](auto& t) {
+    t.n = eng->n; t.k = k; t.idx = idx; t.to_snapshot = to_snapshot ? 1 : 0;
+    launch_snapshot(t, stream);
+  };
+  run(reals);
+  if (words.n_seg) run(words);
+  run(bytes);
+  return launch_check(eng, what, words.n_seg ? 3 : 2);
+}
+
+static int move_envs(CavEngine* eng, const int64_t* idx, int64_t k, void* snap, bool to_snapshot, cudaStream_t stream) {
+  return eng->dtype == CAV_F64 ? move_envs(eng, eng->buf64, idx, k, (char*)snap, to_snapshot, stream)
+                               : move_envs(eng, eng->buf32, idx, k, (char*)snap, to_snapshot, stream);
+}
+
 extern "C" {
 
 const char* cavgym_last_error(void) { return g_error.c_str(); }
@@ -658,6 +761,7 @@ int cavgym_create(const CavScenario* tables, int64_t n_envs, int dtype, int devi
   if (tables->n_spawns > 0) eng->spawns.assign(tables->spawns, tables->spawns + tables->n_spawns);
   eng->host.bodies = eng->bodies.data();
   eng->host.spawns = eng->spawns.data();
+  eng->fingerprint = scenario_fingerprint(eng->host);
   for (const CavBody& body : eng->bodies) {
     if (body.agent == CAV_AGENT_EXTERNAL) eng->has_external = true; else eng->has_device_agents = true;
   }
@@ -701,6 +805,7 @@ int cavgym_destroy(CavEngine* eng) {
   cudaSetDevice(eng->device);
   cudaDeviceSynchronize();
   for (void* p : eng->allocations) cudaFree(p);
+  if (eng->d_stage) cudaFree(eng->d_stage);
   for (cudaStream_t s : eng->pipe) if (s) cudaStreamDestroy(s);
   delete eng;
   return CAV_OK;
@@ -967,6 +1072,105 @@ int cavgym_info(CavEngine* eng, void* polygons_out, void* road_angle_out, cudaSt
     info_kernel<float><<<grid, 128, 0, stream>>>(eng->sc32, eng->tb32, eng->buf32, (const Quad<float>*)eng->d_static_quads,
                                                  (float*)polygons_out, (float*)road_angle_out);
   return launch_check(eng, "info kernel");
+}
+
+int cavgym_snapshot_layout(CavEngine* eng, int64_t k, CavSnapshotLayout* out) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!out || k < 0) return fail(CAV_EINVAL, "out is NULL or k < 0");
+  snapshot_layout(eng, k, out);
+  return CAV_OK;
+}
+
+// The kernels read and write a snapshot in 8-byte (fp64 reals) and, for all envs in order, 16-byte words.
+static int check_snapshot(const void* snapshot) {
+  if (!snapshot) return fail(CAV_EINVAL, "snapshot is NULL");
+  if (reinterpret_cast<uintptr_t>(snapshot) & 15u) return fail(CAV_EINVAL, "snapshot is not 16-byte aligned");
+  return CAV_OK;
+}
+
+int cavgym_save_envs(CavEngine* eng, const int64_t* envs, int64_t k, void* snapshot, cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (k < 0) return fail(CAV_EINVAL, "k < 0");
+  if (k == 0) return CAV_OK;   // an empty selection (whose device pointer may well be NULL) moves nothing
+  if (!envs && k != eng->n) return fail(CAV_EINVAL, "envs is NULL and k is not the engine's env count");
+  if ((rc = check_snapshot(snapshot))) return rc;
+  return move_envs(eng, envs, k, snapshot, true, stream);
+}
+
+int cavgym_load_envs(CavEngine* eng, const int64_t* envs, int64_t k, const void* snapshot, cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (k < 0) return fail(CAV_EINVAL, "k < 0");
+  if (k == 0) return CAV_OK;
+  if (!envs && k != eng->n) return fail(CAV_EINVAL, "envs is NULL and k is not the engine's env count");
+  if (k > eng->n) return fail(CAV_EINVAL, "more target envs than the engine holds: targets must be unique");
+  if ((rc = check_snapshot(snapshot))) return rc;
+  return move_envs(eng, envs, k, const_cast<void*>(snapshot), false, stream);
+}
+
+int cavgym_fork_envs(CavEngine* eng, const int64_t* src, const int64_t* dst, int64_t k, cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (k < 0) return fail(CAV_EINVAL, "k < 0");
+  if (k == 0) return CAV_OK;
+  if (!src || !dst) return fail(CAV_EINVAL, "src/dst is NULL");
+  if (k > eng->n) return fail(CAV_EINVAL, "more target envs than the engine holds: targets must be unique");
+  CavSnapshotLayout L;
+  snapshot_layout(eng, k, &L);
+  if ((size_t)L.total_bytes > eng->stage_bytes) {
+    CUDA_TRY(cudaDeviceSynchronize());   // an earlier fork may still be reading the old staging buffer
+    if (eng->d_stage) CUDA_TRY(cudaFree(eng->d_stage));
+    eng->d_stage = nullptr;
+    eng->stage_bytes = 0;
+    CUDA_TRY(cudaMalloc(&eng->d_stage, (size_t)L.total_bytes));
+    eng->stage_bytes = (size_t)L.total_bytes;
+  }
+  // every read (the gather into the staging snapshot) precedes every write: src may overlap dst and repeat
+  if ((rc = move_envs(eng, src, k, eng->d_stage, true, stream))) return rc;
+  return move_envs(eng, dst, k, eng->d_stage, false, stream);
+}
+
+int cavgym_save_engine(CavEngine* eng, CavEngineState* out) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!out) return fail(CAV_EINVAL, "out is NULL");
+  std::memset(out, 0, sizeof(*out));
+  out->version = CAV_SNAPSHOT_VERSION;
+  out->dtype = eng->dtype;
+  out->m = eng->m;
+  out->n = eng->n;
+  out->shard = eng->buf64.shard;
+  out->t_global = eng->t_global;
+  out->seed = eng->seed;
+  out->fingerprint = eng->fingerprint;
+  out->tau = eng->tau;
+  CUDA_TRY(cudaDeviceSynchronize());
+  const unsigned long long* stats = eng->dtype == CAV_F64 ? eng->buf64.stats : eng->buf32.stats;
+  CUDA_TRY(cudaMemcpy(out->counters, stats, sizeof(out->counters), cudaMemcpyDeviceToHost));
+  return CAV_OK;
+}
+
+int cavgym_load_engine(CavEngine* eng, const CavEngineState* in) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!in) return fail(CAV_EINVAL, "in is NULL");
+  if (in->version != CAV_SNAPSHOT_VERSION) return fail(CAV_EINVAL, "engine state of another version");
+  if (in->fingerprint != eng->fingerprint) return fail(CAV_EINVAL, "engine state of another scenario (fingerprint)");
+  if (in->dtype != eng->dtype || in->m != eng->m || in->n != eng->n)
+    return fail(CAV_EINVAL, "engine state of another dtype, body count or env count");
+  if (in->seed != eng->seed || in->shard != eng->buf64.shard) return fail(CAV_EINVAL, "engine state of another seed or shard");
+  if (!(in->tau >= 0)) return fail(CAV_EINVAL, "tau must be >= 0");
+  CUDA_TRY(cudaDeviceSynchronize());   // the counters and (for another tau) the tables are rewritten under no running kernel
+  const unsigned long long* stats = eng->dtype == CAV_F64 ? eng->buf64.stats : eng->buf32.stats;
+  CUDA_TRY(cudaMemcpy((void*)stats, in->counters, sizeof(in->counters), cudaMemcpyHostToDevice));
+  eng->t_global = in->t_global;
+  if (in->tau != eng->tau) {
+    eng->tau = in->tau;
+    return rebuild_tables(eng);
+  }
+  return CAV_OK;
 }
 
 int cavgym_stats(CavEngine* eng, int64_t* out10 /* [CAV_N_STATS] */) {

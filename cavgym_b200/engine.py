@@ -36,6 +36,59 @@ def _is_float32(array):
     return array is not None and (array.dtype == torch.float32 if isinstance(array, torch.Tensor) else getattr(array, "dtype", None) == np.float32)
 
 
+_REALS = {_abi.CAV_F64: torch.float64, _abi.CAV_F32: torch.float32}
+# (name, section, first row, rows per body or None for one row per env) in the order of CavSnapshotLayout's sections
+_SECTIONS = (("state", "real", 0, 4), ("action", "real", 4, 2), ("agent", "real", 6, _abi.CAV_AGENT_WORDS),
+             ("cs", "real", 6 + _abi.CAV_AGENT_WORDS, 2), ("liveness", "i32", 0, 1), ("t_ep", "i32", 0, None),
+             ("episode", "i32", 1, None), ("winner", "i32", 2, None), ("active", "i32", 3, None), ("done", "u8", 0, None),
+             ("err", "u8", 1, None))
+
+
+class EnvSnapshot:
+    """Everything the kernels keep for k environments, as one uint8 blob (`data`, on any device) laid out by the engine's
+    CavSnapshotLayout (`layout`).  `snap[name]` is a view of one part for inspection: "state" [M,4,K], "action" [M,2,K],
+    "agent" [M,5,K], "cs" [M,2,K] (cos/sin of each heading), "liveness" [M,K], "t_ep", "episode", "winner", "active",
+    "done", "err" [K].  Loading edited rows is unsupported (the cs rows would no longer match the headings): new states go
+    through BatchedCAVEnv.reset(init_state=...)."""
+
+    NAMES = tuple(name for name, *_ in _SECTIONS)
+
+    def __init__(self, data, layout):
+        self.data, self.layout = data, layout
+
+    @property
+    def k(self):
+        return int(self.layout.k)
+
+    @property
+    def device(self):
+        return self.data.device
+
+    def __getitem__(self, name):
+        for key, section, first, per_body in _SECTIONS:
+            if key == name:
+                break
+        else:
+            raise KeyError(f"{name!r} is not one of {self.NAMES}")
+        lay, m, k = self.layout, int(self.layout.m), self.k
+        dtype = {"real": _REALS[lay.dtype], "i32": torch.int32, "u8": torch.uint8}[section]
+        offset = {"real": lay.real_offset, "i32": lay.i32_offset, "u8": lay.u8_offset}[section]
+        rows = {"real": lay.real_rows, "i32": lay.i32_rows, "u8": lay.u8_rows}[section]
+        size = dtype.itemsize
+        table = self.data[offset:offset + rows * k * size].view(dtype).view(rows, k)
+        if per_body is None:
+            return table[first + (m if section == "i32" else 0)]   # the int32 section starts with liveness [M]
+        if section == "i32":
+            return table[:m]
+        return table[first * m:(first + per_body) * m].view(m, per_body, k)
+
+    def to(self, device):
+        return EnvSnapshot(self.data.to(device), self.layout)
+
+    def cpu(self):
+        return self.to("cpu")
+
+
 def _require_cuda(device):
     if not torch.cuda.is_available():
         raise RuntimeError("cavgym_b200 needs a CUDA device (B200, sm_100a); there is no CPU path")
@@ -222,6 +275,121 @@ class BatchedCAVEnv:
                "road_angles": torch.empty((m, n), dtype=self.dtype, device=self.device) if road_angles else None}
         _native.check(self._lib.cavgym_info(self._handle, _ptr(out["body_polygons"]), _ptr(out["road_angles"]), self._stream()))
         return out
+
+    # ---- snapshots: save, restore and fork environments; checkpoint the engine ------------------
+    # The reference-side equivalent is copy.deepcopy(CAVEnv).  Save, load and fork never touch the counters of stats():
+    # an overwritten episode is neither scored nor counted as abandoned, so callers that resample (splitting schemes) keep
+    # their own accounting.  An env's random stream is keyed by (global env id, kind, body, episode, t): an env loaded into
+    # the slot of the same global id (env_offset + index) continues bit for bit, a copy in another slot continues from the
+    # same situation on that slot's own stream.  t_global is batch-wide: a loaded env times out at THIS engine's t_global.
+    def _layout(self, k):
+        layout = _abi.CavSnapshotLayout()
+        _native.check(self._lib.cavgym_snapshot_layout(self._handle, int(k), C.byref(layout)))
+        return layout
+
+    def _indices(self, envs, name, unique=False):
+        """envs (int, list, array or tensor of env indices) as a contiguous int64 device tensor, checked before any launch."""
+        idx = torch.as_tensor(envs, device=self.device)
+        if idx.numel() and (idx.dtype == torch.bool or idx.is_floating_point() or idx.is_complex()):   # [] is float32
+            raise ValueError(f"{name} must hold integer env indices, not {idx.dtype}")
+        idx = idx.reshape(-1).to(torch.int64).contiguous()
+        if idx.numel():
+            n = self.num_envs
+            bad = ((idx < 0) | (idx >= n)).any()
+            repeated = torch.zeros((), dtype=torch.bool, device=self.device)
+            if unique:   # counted on clamped indices: an out-of-range one is reported as such, never used to index
+                counts = torch.zeros(n, dtype=torch.int32, device=self.device)
+                counts.index_add_(0, idx.clamp(0, n - 1), torch.ones_like(idx, dtype=torch.int32))
+                repeated = counts.max() > 1
+            bad, repeated = torch.stack([bad, repeated]).tolist()
+            if bad:
+                raise ValueError(f"{name}: env index outside [0, {n})")
+            if repeated:
+                raise ValueError(f"{name}: repeated target env (targets must be unique)")
+        return idx
+
+    def save_envs(self, envs=None):
+        """EnvSnapshot of the envs listed in `envs` (all, in order, when None) on this engine's device.  Indices may repeat."""
+        idx = None if envs is None else self._indices(envs, "envs")
+        k = self.num_envs if idx is None else idx.numel()
+        layout = self._layout(k)
+        data = torch.empty(int(layout.total_bytes), dtype=torch.uint8, device=self.device)
+        _native.check(self._lib.cavgym_save_envs(self._handle, _ptr(idx), k, _ptr(data), self._stream()))
+        return EnvSnapshot(data, layout)
+
+    def load_envs(self, snapshot, envs=None):
+        """Env envs[j] (env j when envs is None) becomes the snapshot's env j.  Targets must be unique.  The snapshot must
+        come from an engine of the same scenario, dtype and body count (ValueError otherwise)."""
+        if not isinstance(snapshot, EnvSnapshot):
+            raise ValueError("snapshot must be an EnvSnapshot (BatchedCAVEnv.save_envs)")
+        lay = snapshot.layout
+        mine = self._layout(snapshot.k)
+        if lay.version != mine.version:
+            raise ValueError(f"snapshot of layout version {lay.version}, this engine reads version {mine.version}")
+        if lay.fingerprint != mine.fingerprint:
+            raise ValueError("snapshot of another scenario (fingerprint differs)")
+        if lay.dtype != mine.dtype or lay.m != mine.m:
+            raise ValueError(f"snapshot of dtype {_REALS[lay.dtype]} with {lay.m} bodies; this engine: {self.dtype}, {mine.m} bodies")
+        if tuple(snapshot.data.shape) != (int(mine.total_bytes),) or snapshot.data.dtype != torch.uint8:
+            raise ValueError("snapshot data does not have the size its layout gives")
+        idx = None if envs is None else self._indices(envs, "envs", unique=True)
+        k = self.num_envs if idx is None else idx.numel()
+        if k != snapshot.k:
+            raise ValueError(f"snapshot holds {snapshot.k} envs, {k} targets given")
+        data = snapshot.data.to(self.device).contiguous()
+        if data.data_ptr() % 16:   # the kernels read the snapshot in 8- and 16-byte words
+            raise ValueError("snapshot data must start on 16 bytes (a view at an offset is not)")
+        _native.check(self._lib.cavgym_load_envs(self._handle, _ptr(idx), k, _ptr(data), self._stream()))
+
+    def fork(self, src, dst):
+        """Env dst[j] becomes a copy of env src[j].  Every source is read before any target is written, so src may repeat
+        and overlap dst (a population resample); dst must be unique.  A single source is copied into every target.
+        All forks of this engine share one staging snapshot: issue them on one stream.  A fork of more envs than any
+        before it grows that snapshot and synchronises the device."""
+        src_t, dst_t = self._indices(src, "src"), self._indices(dst, "dst", unique=True)
+        if src_t.numel() == 1 and dst_t.numel() > 1:
+            src_t = src_t.expand(dst_t.numel()).contiguous()
+        if src_t.numel() != dst_t.numel():
+            raise ValueError(f"src has {src_t.numel()} envs, dst {dst_t.numel()}")
+        _native.check(self._lib.cavgym_fork_envs(self._handle, _ptr(src_t), _ptr(dst_t), dst_t.numel(), self._stream()))
+
+    def _engine_state(self):
+        state = _abi.CavEngineState()
+        _native.check(self._lib.cavgym_save_engine(self._handle, C.byref(state)))
+        return state
+
+    def state_dict(self):
+        """Checkpoint of the whole engine: every env (as CPU bytes), t_global, the raw counters, seed, shard, tau and the
+        scenario fingerprint.  Tensors, ints, floats and strings only (torch.load with weights_only reads it).  The
+        episode-log ring is not included: drain it first."""
+        state = self._engine_state()
+        envs = self.save_envs().cpu()
+        return {"version": int(state.version), "dtype": str(self.dtype).replace("torch.", ""), "num_envs": int(state.n),
+                "num_bodies": int(state.m), "seed": int(state.seed), "env_offset": int(state.shard), "tau": float(state.tau),
+                "t_global": int(state.t_global), "counters": torch.tensor(list(state.counters), dtype=torch.int64),
+                "fingerprint": f"{state.fingerprint:016x}", "envs": envs.data}
+
+    def load_state_dict(self, state_dict):
+        """Continue a checkpoint of state_dict(): this engine must have the same scenario, dtype, env count, seed and
+        env_offset (ValueError otherwise); tau is taken from the checkpoint."""
+        sd, mine = state_dict, self._engine_state()
+        want = {"version": int(mine.version), "fingerprint": f"{mine.fingerprint:016x}",
+                "dtype": str(self.dtype).replace("torch.", ""), "num_envs": int(mine.n), "num_bodies": int(mine.m),
+                "seed": int(mine.seed), "env_offset": int(mine.shard)}
+        for key, value in want.items():
+            if sd.get(key) != value:
+                raise ValueError(f"checkpoint {key} is {sd.get(key)!r}, this engine has {value!r}")
+        state = _abi.CavEngineState.from_buffer_copy(mine)
+        state.t_global, state.tau = int(sd["t_global"]), float(sd["tau"])
+        counters = [int(v) for v in torch.as_tensor(sd["counters"]).tolist()]
+        if len(counters) != _abi.CAV_N_STATS:
+            raise ValueError(f"checkpoint has {len(counters)} counters, not {_abi.CAV_N_STATS}")
+        state.counters[:] = counters
+        snapshot = EnvSnapshot(torch.as_tensor(sd["envs"]), self._layout(self.num_envs))
+        if tuple(snapshot.data.shape) != (int(snapshot.layout.total_bytes),) or snapshot.data.dtype != torch.uint8:
+            raise ValueError("checkpoint envs do not have the size this engine's layout gives")
+        _native.check(self._lib.cavgym_load_engine(self._handle, C.byref(state)))
+        self.load_envs(snapshot)
 
     # ---- accounting and knobs ------------------------------------------------------------
     def stats(self):

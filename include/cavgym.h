@@ -147,6 +147,32 @@ enum { CAV_STAT_EPISODES = 0, CAV_STAT_INTERESTING = 1, CAV_STAT_SUM_T = 2, CAV_
        CAV_STAT_TANGENT = 8, CAV_STAT_ERRORS = 9, CAV_STAT_SUM_T_INTERESTING = 10, CAV_STAT_SUM_T2_INTERESTING = 11,
        CAV_N_STATS = 12 };
 
+#define CAV_SNAPSHOT_VERSION 1
+
+/* Layout of a snapshot of k envs (cavgym_save_envs): three sections, each starting on 256 bytes, of rows of k elements
+ * (env j of row r at r * k + j).  Reals (dtype): state [M][4], action [M][2], agent [M][CAV_AGENT_WORDS], cs [M][2] (the
+ * cos/sin heading cache); int32: liveness [M], t_ep, episode, winner, active; u8: done, err.  That is everything the
+ * kernels read or write per env.  fingerprint: 64-bit FNV-1a over the scenario tables' contents (the CavScenario header up
+ * to its pointers, then the spawn and body rows), so two engines of the same scenario agree wherever they were built. */
+typedef struct CavSnapshotLayout {
+  int32_t version, dtype, m, reserved;
+  int64_t k;
+  int64_t real_rows, i32_rows, u8_rows;
+  int64_t real_offset, i32_offset, u8_offset;   /* bytes from the start of the snapshot */
+  int64_t total_bytes;
+  uint64_t fingerprint;
+} CavSnapshotLayout;
+
+/* Engine-wide state of a checkpoint (cavgym_save_engine): the raw device counters (before cavgym_stats adds the steps of
+ * episodes in flight), the batch-wide step counter and what an engine must share with the saved one to continue it. */
+typedef struct CavEngineState {
+  int32_t version, dtype, m, reserved;
+  int64_t n, shard, t_global;
+  uint64_t seed, fingerprint;
+  double tau;
+  int64_t counters[CAV_N_STATS];
+} CavEngineState;
+
 /* ---- lifecycle ------------------------------------------------------------------- */
 
 /* CAVEnv.__init__ x n_envs (environment.py:59-92; Config.setup config.py:272-415).
@@ -224,6 +250,36 @@ int cavgym_reset_host(CavEngine* engine, const uint8_t* mask, const void* init_s
  * road_angle_out device real[M][N]: road_angles — DynamicBody.line_anchor_relative_angle towards the major road's centre line
  *                (bodies.py:206-212), NaN where the reference gives None (the body's box intersects the major road), nullable. */
 int cavgym_info(CavEngine* engine, void* polygons_out, void* road_angle_out, cudaStream_t stream);
+
+/* ---- snapshots: save, restore and fork environments; checkpoint an engine ---------- */
+/* The reference-side equivalent is copy.deepcopy(CAVEnv), whose copies share one MT19937 stream; here an env's random
+ * stream is keyed by (global env id, kind, body, episode, t), so an env loaded into a slot of the same global id continues
+ * bit for bit, and a copy in another slot continues from the same situation on that slot's own stream.
+ * Save, load and fork never touch the counters of cavgym_stats: an overwritten episode is neither scored nor counted as
+ * abandoned.  t_global is batch-wide (cavgym_save_engine), so a loaded env times out at the loading engine's t_global.
+ * Snapshot rows are not meant to be edited: the cs rows must match the headings; new states go through cavgym_reset.
+ * A snapshot is only valid for an engine of the same scenario (fingerprint), dtype and body count.
+ * The kernels are ordinary launches on `stream`; a cavgym_replay that follows waits for them like for any other call. */
+
+/* Layout of a snapshot of k envs of this engine; out is HOST memory. */
+int cavgym_snapshot_layout(CavEngine* engine, int64_t k, CavSnapshotLayout* out);
+/* Copies envs[0..k) (device int64, NULL = all N in order with k = N) into `snapshot` (device, layout total_bytes, 16-byte
+ * aligned: CAV_EINVAL otherwise; cudaMalloc and torch allocations are).  k = 0 does nothing.  Indices outside [0, N) are
+ * skipped. */
+int cavgym_save_envs(CavEngine* engine, const int64_t* envs, int64_t k, void* snapshot, cudaStream_t stream);
+/* Writes snapshot column j into env envs[j] (device int64, unique, NULL = all N in order); snapshot as for
+ * cavgym_save_envs.  k = 0 does nothing. */
+int cavgym_load_envs(CavEngine* engine, const int64_t* envs, int64_t k, const void* snapshot, cudaStream_t stream);
+/* Env dst[j] becomes a copy of env src[j] (device int64, dst unique; src may repeat and overlap dst): every source is read,
+ * into an engine-owned staging snapshot, before any target is written.  k = 0 does nothing.  All forks of one engine share
+ * that staging snapshot, so they must be ordered on one stream.  A fork of more envs than any fork before it on the engine
+ * grows the staging snapshot, which synchronises the device (and so cannot be captured into a CUDA graph). */
+int cavgym_fork_envs(CavEngine* engine, const int64_t* src, const int64_t* dst, int64_t k, cudaStream_t stream);
+/* Engine-wide state; out is HOST memory.  Synchronises. */
+int cavgym_save_engine(CavEngine* engine, CavEngineState* out);
+/* Restores t_global, the raw counters and tau after checking fingerprint, dtype, m, n, seed and shard (CAV_EINVAL on a
+ * mismatch).  The episode-log ring, the replay launch chain and every knob are not part of the state.  Synchronises. */
+int cavgym_load_engine(CavEngine* engine, const CavEngineState* in);
 
 /* ---- accounting ------------------------------------------------------------------ */
 
