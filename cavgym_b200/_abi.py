@@ -66,6 +66,11 @@ class CavEngineState(C.Structure):
                 ("tau", C.c_double), ("counters", C.c_int64 * CAV_N_STATS)]
 
 
+class CavRolloutRecord(C.Structure):
+    _fields_ = [("observation", C.c_void_p), ("action", C.c_void_p), ("state", C.c_void_p), ("reward", C.c_void_p),
+                ("done", C.c_void_p), ("winner", C.c_void_p), ("tangent", C.c_void_p), ("timestep", C.c_void_p)]
+
+
 class CavScenario(C.Structure):
     _fields_ = [("n_bodies", C.c_int32), ("n_types", C.c_int32), ("n_roads", C.c_int32), ("n_statics", C.c_int32),
                 ("n_spawns", C.c_int32), ("terminate_collisions", C.c_int32), ("terminate_ego_zones", C.c_int32),
@@ -89,6 +94,7 @@ PROTOTYPES = {
     "cavgym_reset": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, c_stream]),
     "cavgym_step": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
     "cavgym_rollout": (C.c_int, [c_engine_p, C.c_int, C.c_int, c_stream]),
+    "cavgym_rollout_record": (C.c_int, [c_engine_p, C.c_int, C.c_int, C.POINTER(CavRolloutRecord), c_stream]),
     "cavgym_replay": (C.c_int, [c_engine_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
     "cavgym_step_host": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cavgym_step_host_f32": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -138,6 +138,21 @@ struct StepIO {
   int32_t seq, chained;
 };
 
+// cavgym_rollout_record: the per-step [T] slabs of a recorded rollout (CavRolloutRecord), each nullable; row t of a slab
+// has the per-step shape with the env index fastest.  Only the recording kernels take it, so StepIO, EnvBuffers and
+// DevScenario — parameters of every kernel — keep their layout.
+template <typename R>
+struct RolloutRecord {
+  R* observation;      // [T][M][4][N] state the agents saw at step t (after the auto-reset)
+  R* action;           // [T][M][2][N] joint action executed at step t
+  R* state;            // [T][M][4][N] state after step t
+  R* reward;           // [T][M][N]
+  uint8_t* done;       // [T][N]
+  int32_t* winner;     // [T][N]
+  uint8_t* tangent;    // [T][N]
+  int32_t* timestep;   // [T][N] t_ep after step t, 0 where the env did not step
+};
+
 // cavgym_step_host_f32: joint actions and results cross the host link as float32 while the engine steps in its own type.
 struct WireIO32 {
   const float* actions;  // [M][2][N]

@@ -28,7 +28,9 @@ namespace cav {
 #define CAV_FOR_EACH_M(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8)
 #define CAV_DECLARE(K)                                   \
   extern const SmallLaunchers<double> kSmallF64M##K;     \
-  extern const SmallLaunchers<float> kSmallF32M##K;
+  extern const SmallLaunchers<float> kSmallF32M##K;      \
+  extern const RolloutRecordLauncher<double> kRecordF64M##K; \
+  extern const RolloutRecordLauncher<float> kRecordF32M##K;
 CAV_FOR_EACH_M(CAV_DECLARE)
 #undef CAV_DECLARE
 
@@ -43,6 +45,23 @@ template <> const SmallLaunchers<double>* small_launchers<double>(int m) {
 template <> const SmallLaunchers<float>* small_launchers<float>(int m) {
   switch (m) {
 #define CAV_CASE(K) case K: return &kSmallF32M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+
+template <> RolloutRecordLauncher<double> rollout_record_launcher<double>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kRecordF64M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+template <> RolloutRecordLauncher<float> rollout_record_launcher<float>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kRecordF32M##K;
     CAV_FOR_EACH_M(CAV_CASE)
 #undef CAV_CASE
     default: return nullptr;
@@ -699,6 +718,20 @@ static int move_envs(CavEngine* eng, const int64_t* idx, int64_t k, void* snap, 
                                : move_envs(eng, eng->buf32, idx, k, (char*)snap, to_snapshot, stream);
 }
 
+// ---------------------------------------------------------------- recorded rollouts
+template <typename R>
+static int rollout_record_typed(CavEngine* eng, const DevScenario<R>& sc, const EnvBuffers<R>& buf, const CavRolloutRecord& r,
+                                int n_steps, int auto_reset, cudaStream_t stream) {
+  const RolloutRecord<R> rec{(R*)r.observation, (R*)r.action, (R*)r.state, (R*)r.reward, r.done, r.winner, r.tangent, r.timestep};
+  if (eng->dense) {
+    if (!dense_launchers<R>()->rollout_record(sc, dense_tables<R>(eng), buf, rec, eng->t_global, n_steps, auto_reset, stream))
+      return fail(CAV_ECUDA, "dense kernel set-up failed (shared memory opt-in)");
+    return launch_check(eng, "dense record kernel");
+  }
+  rollout_record_launcher<R>(eng->m)(sc, buf, rec, eng->t_global, n_steps, auto_reset, stream);   // also for eng->team
+  return launch_check(eng, "rollout record kernel");
+}
+
 extern "C" {
 
 const char* cavgym_last_error(void) { return g_error.c_str(); }
@@ -878,6 +911,21 @@ int cavgym_rollout(CavEngine* eng, int n_steps, int auto_reset, cudaStream_t str
     else small_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
   }
   rc = launch_check(eng, "rollout kernel");
+  if (rc) return rc;
+  eng->t_global += n_steps;
+  return CAV_OK;
+}
+
+int cavgym_rollout_record(CavEngine* eng, int n_steps, int auto_reset, const CavRolloutRecord* rec, cudaStream_t stream) {
+  if (!rec || !(rec->observation || rec->action || rec->state || rec->reward || rec->done || rec->winner || rec->tangent || rec->timestep))
+    return cavgym_rollout(eng, n_steps, auto_reset, stream);
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (n_steps < 0) return fail(CAV_EINVAL, "n_steps must be >= 0");
+  if (eng->has_external) return fail(CAV_ESTATE, "cavgym_rollout_record needs an on-device agent for every body");
+  if (n_steps == 0) return CAV_OK;
+  rc = eng->dtype == CAV_F64 ? rollout_record_typed(eng, eng->sc64, eng->buf64, *rec, n_steps, auto_reset, stream)
+                             : rollout_record_typed(eng, eng->sc32, eng->buf32, *rec, n_steps, auto_reset, stream);
   if (rc) return rc;
   eng->t_global += n_steps;
   return CAV_OK;

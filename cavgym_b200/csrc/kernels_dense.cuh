@@ -359,10 +359,11 @@ __device__ __noinline__ bool dense_pair(const DenseSmem<R>& sm, const DenseTable
 
 // One joint transition of env e by its warp.  `actions` = this step's [M][2][N] rows (nullable when every body has an
 // on-device agent).  Returns with env updated; outputs written through `io`.
-template <typename R, bool AGENTS>
+// RECORD (dense_record_kernel): `act_rec` (nullable) receives this step's [M][2][N] joint action row.
+template <typename R, bool AGENTS, bool RECORD = false>
 __device__ __forceinline__ void dense_transition(const DevScenario<R>& sc, const DenseTables<R>& tb, const EnvBuffers<R>& buf,
                                                  const StepIO<R>& io, const R* actions, int64_t e, int64_t t_global, int lane,
-                                                 const DenseSmem<R>& sm, DenseEnv& env, const bool phase_sync) {
+                                                 const DenseSmem<R>& sm, DenseEnv& env, const bool phase_sync, R* act_rec = nullptr) {
   const int M = sc.n_bodies, Mp = (M + 31) & ~31;
   const int64_t n = buf.n;
   const R tau = sc.tau, dt = sc.dt;
@@ -511,6 +512,9 @@ __device__ __forceinline__ void dense_transition(const DevScenario<R>& sc, const
     if (io.state_out && io.state_out != buf.state) {
 #pragma unroll
       for (int w = 0; w < 4; ++w) io.state_out[((int64_t)b * 4 + w) * n + e] = st[w];
+    }
+    if constexpr (RECORD) {
+      if (act_rec) { act_rec[((int64_t)b * 2 + 0) * n + e] = a0; act_rec[((int64_t)b * 2 + 1) * n + e] = a1; }
     }
   }
   __syncwarp();
@@ -820,6 +824,90 @@ __global__ void __launch_bounds__(kDenseWarps * 32, CAV_DENSE_MIN_BLOCKS) dense_
   else dense_writeback_env<R>(sc, buf, e, lane, sm, env);
 }
 
+// cavgym_rollout_record on the warp-per-env path: dense_kernel<R, true>'s loop with traj = 1 (io = rec's state, reward, done,
+// winner and tangent slabs) that also writes the observation before each step's transition, the executed action and t_ep
+// after it; frozen rows get the frozen state, action 0 and timestep 0.  A kernel of its own so that dense_kernel's code
+// stays as it is.
+template <typename R>
+__global__ void __launch_bounds__(kDenseWarps * 32, CAV_DENSE_MIN_BLOCKS) dense_record_kernel(const __grid_constant__ DevScenario<R> sc,
+                                                                        const __grid_constant__ DenseTables<R> tb,
+                                                                        const __grid_constant__ EnvBuffers<R> buf,
+                                                                        const __grid_constant__ StepIO<R> io,
+                                                                        const __grid_constant__ RolloutRecord<R> rec, int64_t t_global,
+                                                                        int n_steps, int auto_reset) {
+  extern __shared__ __align__(16) unsigned char dense_smem[];
+  const int M = sc.n_bodies, Mp = (M + 31) & ~31;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  float4* bp_all = reinterpret_cast<float4*>(dense_smem);
+  R* geo_all = reinterpret_cast<R*>(dense_smem + sizeof(float4) * kDenseWarps * (Mp + kDenseTiles));
+  int32_t* meta = reinterpret_cast<int32_t*>(geo_all + (size_t)kDenseWarps * 6 * Mp);
+  for (int b = threadIdx.x; b < Mp; b += blockDim.x) meta[b] = b < M ? tb.bodies[b].meta : (int32_t)DM_ABSENT;
+  __syncthreads();
+  const int64_t e = buf.lo + (int64_t)blockIdx.x * kDenseWarps + warp;
+  const bool phase_sync = CAV_DENSE_SYNC >= 2 && auto_reset && !tb.has_external;
+  if (e >= buf.hi) {   // a warp of the ragged last CTA without an env: keep the barriers below balanced
+    if (CAV_DENSE_SYNC) for (int t = 0; t < n_steps * (phase_sync ? 3 : 1); ++t) __syncthreads();
+    return;
+  }
+  DenseSmem<R> sm;
+  sm.bp = bp_all + (size_t)warp * (Mp + kDenseTiles);
+  sm.tu = sm.bp + Mp;
+  R* geo = geo_all + (size_t)warp * 6 * Mp;
+  sm.x = geo; sm.y = geo + Mp; sm.v = geo + 2 * Mp; sm.c = geo + 3 * Mp; sm.s = geo + 4 * Mp; sm.th = geo + 5 * Mp;
+  sm.meta = meta;
+  const int64_t n = buf.n;
+
+  DenseEnv env;
+  env.done = buf.done[e];
+  env.t_ep = buf.t_ep[e];
+  env.winner = env.done ? buf.winner[e] : -1;
+  env.episode = buf.episode[e];
+  dense_stage_env<R, true>(sc, buf, e, lane, sm, env);
+  for (int t = 0; t < n_steps; ++t) {
+    if (CAV_DENSE_SYNC) __syncthreads();
+    const StepIO<R> at = io_at(io, (int64_t)t, (int64_t)M, n);
+    const int64_t row = (int64_t)t * n;
+    R* act = rec.action ? rec.action + row * M * 2 : nullptr;
+    if (env.done && auto_reset) {
+      dense_reset_env<R>(sc, tb, buf, nullptr, e, lane, env);
+      dense_stage_env<R, true>(sc, buf, e, lane, sm, env);
+    }
+    for (int b = lane; b < M; b += 32) {   // lane-private bodies: staged and stepped by this lane
+      if (rec.observation) {
+        R* o = rec.observation + row * M * 4;
+        o[((int64_t)b * 4 + 0) * n + e] = sm.x[b];
+        o[((int64_t)b * 4 + 1) * n + e] = sm.y[b];
+        o[((int64_t)b * 4 + 2) * n + e] = sm.v[b];
+        o[((int64_t)b * 4 + 3) * n + e] = sm.th[b];
+      }
+      if (env.done && act) { act[((int64_t)b * 2 + 0) * n + e] = R(0); act[((int64_t)b * 2 + 1) * n + e] = R(0); }
+    }
+    if (env.done) {   // frozen until reset: reward 0, latched done / winner, timestep 0
+      for (int b = lane; b < M; b += 32) {
+        if (at.reward_out) at.reward_out[(int64_t)b * n + e] = R(0);
+        if (at.state_out) {
+          at.state_out[((int64_t)b * 4 + 0) * n + e] = sm.x[b];
+          at.state_out[((int64_t)b * 4 + 1) * n + e] = sm.y[b];
+          at.state_out[((int64_t)b * 4 + 2) * n + e] = sm.v[b];
+          at.state_out[((int64_t)b * 4 + 3) * n + e] = sm.th[b];
+        }
+      }
+      if (lane == 0) {
+        if (at.done_out) at.done_out[e] = env.done == 1 ? 1 : 0;
+        if (at.winner_out) at.winner_out[e] = env.winner;
+        if (at.tangent_out) at.tangent_out[e] = 0;
+        if (rec.timestep) rec.timestep[row + e] = 0;
+      }
+      continue;
+    }
+    dense_transition<R, true, true>(sc, tb, buf, at, nullptr, e, t_global + t, lane, sm, env, phase_sync, act);
+    if (lane == 0 && rec.timestep) rec.timestep[row + e] = env.t_ep;
+    __syncwarp();
+  }
+  if (auto_reset && env.done) dense_reset_env<R>(sc, tb, buf, nullptr, e, lane, env);
+  else dense_writeback_env<R>(sc, buf, e, lane, sm, env);
+}
+
 template <typename R>
 __global__ void __launch_bounds__(kDenseWarps * 32) dense_reset_kernel(const __grid_constant__ DevScenario<R> sc,
                                                                        const __grid_constant__ DenseTables<R> tb,
@@ -847,6 +935,9 @@ struct DenseLaunchers {
               int auto_reset, int traj, bool agents, cudaStream_t);
   void (*reset)(const DevScenario<R>&, const DenseTables<R>&, const EnvBuffers<R>&, const uint8_t* mask, const R* init, int first_time,
                 cudaStream_t);
+  // cavgym_rollout_record; false = launch set-up failed
+  bool (*rollout_record)(const DevScenario<R>&, const DenseTables<R>&, const EnvBuffers<R>&, const RolloutRecord<R>&, int64_t t_global,
+                         int n_steps, int auto_reset, cudaStream_t);
 };
 
 template <typename R, bool AGENTS>
@@ -866,6 +957,19 @@ bool launch_dense(const DevScenario<R>& sc, const DenseTables<R>& tb, const EnvB
                   int n_steps, int auto_reset, int traj, bool agents, cudaStream_t stream) {
   return agents ? launch_dense_typed<R, true>(sc, tb, buf, io, t_global, n_steps, auto_reset, traj, stream)
                 : launch_dense_typed<R, false>(sc, tb, buf, io, t_global, n_steps, auto_reset, traj, stream);
+}
+
+template <typename R>
+bool launch_dense_record(const DevScenario<R>& sc, const DenseTables<R>& tb, const EnvBuffers<R>& buf, const RolloutRecord<R>& rec,
+                         int64_t t_global, int n_steps, int auto_reset, cudaStream_t stream) {
+  const size_t smem = dense_smem_bytes<R>(sc.n_bodies, kDenseWarps);
+  if (smem > 48 * 1024 &&
+      cudaFuncSetAttribute(dense_record_kernel<R>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
+    return false;
+  const StepIO<R> io{nullptr, rec.state, rec.reward, rec.done, rec.winner, rec.tangent, 0};
+  const unsigned grid = (unsigned)((buf.hi - buf.lo + kDenseWarps - 1) / kDenseWarps);
+  dense_record_kernel<R><<<grid, kDenseWarps * 32, smem, stream>>>(sc, tb, buf, io, rec, t_global, n_steps, auto_reset);
+  return true;
 }
 
 template <typename R>

@@ -3,6 +3,7 @@
 //   step_kernel     one CAVEnv.step over all N envs                 (cavgym_step)
 //   replay_kernel   T steps on replayed joint actions, state kept in registers   (cavgym_replay)
 //   rollout_kernel  T steps with on-device agents, scoring and auto-reset in-kernel  (cavgym_rollout)
+//   rollout_record_kernel  the same, writing per-step [T] slabs                    (cavgym_rollout_record)
 //   reset_kernel    CAVEnv.reset for masked envs                    (cavgym_reset / cavgym_create)
 //
 // HBM layout is SoA with the environment index fastest, so lane i of a warp touches
@@ -304,6 +305,64 @@ __global__ void __launch_bounds__((rollout_threads<GENERIC, M>()), (rollout_min_
   store_env<R, M, true>(sc, buf, e, env, was_reset);
 }
 
+// cavgym_rollout_record: rollout_kernel's loop, writing row t of every slab of `rec` for each env — the observation after
+// the auto-reset at the top of step t, then through advance() the post-step state, reward, done, winner and tangent, then
+// the executed action and t_ep.  An env that does not step (finished, auto_reset = 0) keeps filling its rows as a frozen
+// env (state unchanged, reward 0, latched done / winner, action 0, timestep 0) where rollout_kernel leaves its loop.  Ghost
+// lanes write nothing.  A kernel of its own rather than a flag of rollout_kernel, so that rollout_kernel's code stays as it
+// is; the rewards, which rollout_kernel never stores, are formed only here.
+template <typename R, int M, bool GENERIC>
+__global__ void __launch_bounds__((rollout_threads<GENERIC, M>()), (rollout_min_blocks<GENERIC, M>())) rollout_record_kernel(
+    const __grid_constant__ DevScenario<R> sc, const __grid_constant__ EnvBuffers<R> buf, const __grid_constant__ RolloutRecord<R> rec,
+    int64_t t_global, int n_steps, int auto_reset) {
+  const int64_t e_raw = buf.lo + (int64_t)blockIdx.x * rollout_threads<GENERIC, M>() + threadIdx.x;
+  const bool in_range = e_raw < buf.hi;
+  constexpr bool kSync = (GENERIC && M >= CAV_ROLLOUT_SYNC_FROM_M) || (CAV_ROLLOUT_SYNC_HOMOGENEOUS != 0 && !GENERIC);
+  using Phase = typename std::conditional<kSync, CtaPhase, NoPhase>::type;
+  const bool sync_on = kSync && auto_reset != 0;
+  if (!in_range && !sync_on) return;
+  const bool ghost = !in_range;
+  const int64_t e = in_range ? e_raw : buf.hi - 1;
+  const int64_t n = buf.n;
+  Phase phase;
+  if constexpr (kSync) phase.on = sync_on;
+  EnvRegs<R, M> env;
+  load_env<R, M, true>(sc, buf, e, env);
+  R ext[M][2];
+  load_actions<R, M>(nullptr, n, e, ext);
+  bool was_reset = false;
+  for (int t = 0; t < n_steps; ++t) {
+    if (sync_on) { __syncwarp(); __syncthreads(); }
+    if (CAV_UNLIKELY(env.done != 0) && auto_reset) {
+      reset_env<R, M>(sc, buf, nullptr, e, env);
+      was_reset = true;
+    }
+    const int64_t row = (int64_t)t * n;
+    const bool stepped = env.done == 0;
+    if (!ghost && rec.observation) {
+#pragma unroll
+      for (int b = 0; b < M; ++b)
+#pragma unroll
+        for (int c = 0; c < 4; ++c) rec.observation[row * (M * 4) + ((int64_t)b * 4 + c) * n + e] = env.s[b][c];
+    }
+    const StepIO<R> at = {nullptr, rec.state ? rec.state + row * (M * 4) : nullptr, rec.reward ? rec.reward + row * M : nullptr,
+                          rec.done ? rec.done + row : nullptr, rec.winner ? rec.winner + row : nullptr,
+                          rec.tangent ? rec.tangent + row : nullptr, 0};
+    advance<R, M, true, GENERIC, Phase>(sc, buf, at, e, t_global + t, env, ext, phase, ghost);
+    if (!ghost && rec.action) {
+#pragma unroll
+      for (int b = 0; b < M; ++b) {
+        rec.action[row * (M * 2) + ((int64_t)b * 2 + 0) * n + e] = stepped ? env.held[b][0] : R(0);
+        rec.action[row * (M * 2) + ((int64_t)b * 2 + 1) * n + e] = stepped ? env.held[b][1] : R(0);
+      }
+    }
+    if (!ghost && rec.timestep) rec.timestep[row + e] = stepped ? env.t_ep : 0;
+  }
+  if (ghost) return;
+  if (auto_reset && env.done) { reset_env<R, M>(sc, buf, nullptr, e, env); was_reset = true; }
+  store_env<R, M, true>(sc, buf, e, env, was_reset);
+}
+
 template <typename R, int M>
 __global__ void __launch_bounds__(kThreads) reset_kernel(const __grid_constant__ DevScenario<R> sc,
                                                          const __grid_constant__ EnvBuffers<R> buf, const uint8_t* mask,
@@ -389,6 +448,13 @@ void launch_rollout(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t 
   else rollout_kernel<R, M, true><<<grid_for(buf, synced), synced, 0, stream>>>(sc, buf, t_global, n_steps, auto_reset);
 }
 template <typename R, int M>
+void launch_rollout_record(const DevScenario<R>& sc, const EnvBuffers<R>& buf, const RolloutRecord<R>& rec, int64_t t_global,
+                           int n_steps, int auto_reset, cudaStream_t stream) {
+  constexpr int plain = rollout_threads<false, M>(), synced = rollout_threads<true, M>();
+  if (sc.homogeneous) rollout_record_kernel<R, M, false><<<grid_for(buf, plain), plain, 0, stream>>>(sc, buf, rec, t_global, n_steps, auto_reset);
+  else rollout_record_kernel<R, M, true><<<grid_for(buf, synced), synced, 0, stream>>>(sc, buf, rec, t_global, n_steps, auto_reset);
+}
+template <typename R, int M>
 void launch_reset(const DevScenario<R>& sc, const EnvBuffers<R>& buf, const uint8_t* mask, const R* init, int first_time,
                   cudaStream_t stream) {
   reset_kernel<R, M><<<grid_for(buf), kThreads, 0, stream>>>(sc, buf, mask, init, first_time);
@@ -396,5 +462,12 @@ void launch_reset(const DevScenario<R>& sc, const EnvBuffers<R>& buf, const uint
 
 // Defined in small_mK.cu (one translation unit per body count so they compile in parallel).
 template <typename R> const SmallLaunchers<R>* small_launchers(int m);
+
+// cavgym_rollout_record (launch_rollout_record), defined in record_mK.cu: translation units apart from small_mK.cu, where a
+// further caller of the transition's out-of-line helpers would change how they are compiled for the existing kernels.
+template <typename R>
+using RolloutRecordLauncher = void (*)(const DevScenario<R>&, const EnvBuffers<R>&, const RolloutRecord<R>&, int64_t t_global,
+                                       int n_steps, int auto_reset, cudaStream_t);
+template <typename R> RolloutRecordLauncher<R> rollout_record_launcher(int m);
 
 }  // namespace cav

@@ -180,9 +180,37 @@ class BatchedCAVEnv:
                                             _ptr(self.winner), _ptr(self.tangent), self._stream()))
         return (self.state if copy_state is None else copy_state), self.reward, self.done, self.winner, self.tangent
 
-    def rollout(self, n_steps, auto_reset=True):
-        """Simulation.run's timestep loop with the on-device agents: n_steps fused transitions per launch."""
-        _native.check(self._lib.cavgym_rollout(self._handle, int(n_steps), int(bool(auto_reset)), self._stream()))
+    # field -> (per-step shape as a function of (M, N), dtype: None = the engine's real type)
+    RECORD_FIELDS = {"observation": (lambda m, n: (m, 4, n), None), "action": (lambda m, n: (m, 2, n), None),
+                     "state": (lambda m, n: (m, 4, n), None), "reward": (lambda m, n: (m, n), None),
+                     "done": (lambda m, n: (n,), torch.uint8), "winner": (lambda m, n: (n,), torch.int32),
+                     "tangent": (lambda m, n: (n,), torch.uint8), "timestep": (lambda m, n: (n,), torch.int32)}
+
+    def rollout(self, n_steps, auto_reset=True, record=None):
+        """Simulation.run's timestep loop with the on-device agents: n_steps fused transitions per launch.
+
+        record=None returns None.  A tuple of names from RECORD_FIELDS also records those per-step returns and returns them
+        as a dict of new device tensors [T, ...] in the engine's layout (see cavgym_rollout_record): "observation" [T,M,4,N]
+        (the state the agents saw, after any auto-reset), "action" [T,M,2,N] (the joint action executed), "state" [T,M,4,N]
+        (after the step), "reward" [T,M,N], "done" / "tangent" uint8 [T,N], "winner" / "timestep" int32 [T,N].  A row
+        where an env did not step has timestep 0.  Recording changes nothing else: the engine state, counters, episode-log
+        rows and t_global are those of the same rollout without it.  trajectories.complete_episodes splits a record."""
+        n_steps = int(n_steps)
+        if record is None:
+            _native.check(self._lib.cavgym_rollout(self._handle, n_steps, int(bool(auto_reset)), self._stream()))
+            return None
+        names = (record,) if isinstance(record, str) else tuple(record)
+        unknown = [name for name in names if name not in self.RECORD_FIELDS]
+        if unknown:
+            raise ValueError(f"unknown record field(s) {unknown}; choose from {tuple(self.RECORD_FIELDS)}")
+        if n_steps < 0:
+            raise ValueError("n_steps must be >= 0")
+        m, n = self.num_bodies, self.num_envs
+        out = {name: torch.empty((n_steps,) + shape(m, n), dtype=dtype or self.dtype, device=self.device)
+               for name, (shape, dtype) in self.RECORD_FIELDS.items() if name in names}
+        rec = _abi.CavRolloutRecord(**{name: tensor.data_ptr() for name, tensor in out.items() if tensor.numel()})
+        _native.check(self._lib.cavgym_rollout_record(self._handle, n_steps, int(bool(auto_reset)), C.byref(rec), self._stream()))
+        return out
 
     def replay(self, actions, record=("state", "reward", "done", "winner", "tangent")):
         """Replay joint actions [T,M,2,N] in one launch; returns the recorded trajectories as a dict."""

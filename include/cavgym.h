@@ -213,6 +213,36 @@ int cavgym_step(CavEngine* engine, const void* actions, void* state_out, void* r
  * (reporting.py:227-243) and reset in the same kernel. */
 int cavgym_rollout(CavEngine* engine, int n_steps, int auto_reset, cudaStream_t stream);
 
+/* The per-step returns of env.step inside Simulation.run's loop (simulation.py:38-118), for a cavgym_rollout: device slabs
+ * [T] x the per-step shape, env index fastest (as cavgym_replay's), each nullable.  Row t holds
+ *   observation real[T][M][4][N]  the state the agents saw when they chose step t's actions: AFTER any auto-reset at the top
+ *                                 of step t (the reference's observation, environment.py:223-229)
+ *   action      real[T][M][2][N]  the joint action executed at step t, for every agent kind (what
+ *                                 cavgym_set_action_logging stores)
+ *   state       real[T][M][4][N]  the state after step t
+ *   reward      real[T][M][N], done u8[T][N], winner i32[T][N], tangent u8[T][N]   as cavgym_replay's
+ *   timestep    i32[T][N]         the env's t_ep after step t: 1 on the first step of an episode
+ * A row where the env does not step (finished, auto_reset = 0) is a frozen row, as in cavgym_replay: state and observation
+ * unchanged, reward 0, done / winner latched, tangent 0, action 0, timestep 0.  So an episode starts at a row with
+ * timestep == 1; it ends at a row with done == 1 and timestep > 0, or — cut off at max_timesteps (done stays 0) — at a row
+ * with timestep == max_timesteps. */
+typedef struct CavRolloutRecord {
+  void* observation;
+  void* action;
+  void* state;
+  void* reward;
+  uint8_t* done;
+  int32_t* winner;
+  uint8_t* tangent;
+  int32_t* timestep;
+} CavRolloutRecord;
+
+/* cavgym_rollout that also writes `rec` (HOST struct of device pointers; NULL or all-NULL = cavgym_rollout).  The launches,
+ * engine state, counters, episode-log rows and t_global afterwards are exactly those of cavgym_rollout.  With
+ * cavgym_set_rollout_path(team = 1) a recorded rollout runs the thread-per-environment kernel (the team kernel forms no
+ * rewards); its results are bitwise the same. */
+int cavgym_rollout_record(CavEngine* engine, int n_steps, int auto_reset, const CavRolloutRecord* rec, cudaStream_t stream);
+
 /* Replayed joint actions, n_steps transitions in one launch:
  * actions real[T][M][2][N]; trajectory outputs (each nullable) state real[T][M][4][N],
  * reward real[T][M][N], done u8[T][N], winner i32[T][N], tangent u8[T][N].
