@@ -126,7 +126,6 @@ PROTOTYPES = {
     "cavgym_set_step_path": (C.c_int, [c_engine_p, C.c_int]),
     "cavgym_set_host_path": (C.c_int, [c_engine_p, C.c_int]),
     "cavgym_set_dense_path": (C.c_int, [c_engine_p, C.c_int]),
-    "cavgym_set_rollout_path": (C.c_int, [c_engine_p, C.c_int]),
     "cavgym_set_tangent_tolerance": (C.c_int, [c_engine_p, C.c_double]),
     "cavgym_bodies_step": (C.c_int, [C.POINTER(CavBodyType), C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_int, c_stream]),
     "cavgym_geometry_probe": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_int, c_stream]),

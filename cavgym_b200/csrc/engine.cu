@@ -19,7 +19,6 @@
 #ifndef CAV_REPLAY_CHAIN   // 0: every replay launch waits for the whole previous grid (A/B)
 #define CAV_REPLAY_CHAIN 1
 #endif
-#include "kernels_team.cuh"
 #include "kernels_tma.cuh"   // (tma_span, kReplayTile for the replay launch chain; includes kernels_small.cuh)
 #include "kernels_snapshot.cuh"
 
@@ -433,7 +432,6 @@ struct CavEngine {
   bool has_external = false, has_device_agents = false;
   bool use_tma = true;  // cavgym_set_step_path: 0 = plain thread-per-env kernel only
   bool zero_copy_host = true;  // cavgym_set_host_path: 0 = always stage host buffers through device copies
-  bool team = false;           // cavgym_set_rollout_path: team-of-warps rollout kernels (kernels_team.cuh) where they apply (measured: no faster, DESIGN 4.6)
   bool dense = false;          // warp-per-env kernels (kernels_dense.cuh): always for m > CAV_SMALL_M, cavgym_set_dense_path otherwise
   DenseTables<double> tb64;
   DenseTables<float> tb32;
@@ -728,7 +726,7 @@ static int rollout_record_typed(CavEngine* eng, const DevScenario<R>& sc, const 
       return fail(CAV_ECUDA, "dense kernel set-up failed (shared memory opt-in)");
     return launch_check(eng, "dense record kernel");
   }
-  rollout_record_launcher<R>(eng->m)(sc, buf, rec, eng->t_global, n_steps, auto_reset, stream);   // also for eng->team
+  rollout_record_launcher<R>(eng->m)(sc, buf, rec, eng->t_global, n_steps, auto_reset, stream);
   return launch_check(eng, "rollout record kernel");
 }
 
@@ -899,17 +897,8 @@ int cavgym_rollout(CavEngine* eng, int n_steps, int auto_reset, cudaStream_t str
     eng->t_global += n_steps;
     return CAV_OK;
   }
-  // opt-in (cavgym_set_rollout_path) for heterogeneous scenarios of three bodies or more: a team of warps, one per body
-  // (kernels_team.cuh); everything else — and election agents — thread per env
-  bool launched = false;
-  if (eng->team) {
-    launched = eng->dtype == CAV_F64 ? team_launchers<double>()->rollout(eng->sc64, eng->buf64, eng->t_global, n_steps, auto_reset, stream)
-                                     : team_launchers<float>()->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
-  }
-  if (!launched) {
-    if (eng->dtype == CAV_F64) small_launchers<double>(eng->m)->rollout(eng->sc64, eng->buf64, eng->t_global, n_steps, auto_reset, stream);
-    else small_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
-  }
+  if (eng->dtype == CAV_F64) small_launchers<double>(eng->m)->rollout(eng->sc64, eng->buf64, eng->t_global, n_steps, auto_reset, stream);
+  else small_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
   rc = launch_check(eng, "rollout kernel");
   if (rc) return rc;
   eng->t_global += n_steps;
@@ -1335,12 +1324,6 @@ int cavgym_set_action_logging(CavEngine* eng, int enabled) {
 int cavgym_set_step_path(CavEngine* eng, int use_tma) {
   if (!eng) return fail(CAV_EINVAL, "engine is NULL");
   eng->use_tma = use_tma != 0;
-  return CAV_OK;
-}
-
-int cavgym_set_rollout_path(CavEngine* eng, int team) {
-  if (!eng) return fail(CAV_EINVAL, "engine is NULL");
-  eng->team = team != 0;
   return CAV_OK;
 }
 

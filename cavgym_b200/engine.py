@@ -453,11 +453,6 @@ class BatchedCAVEnv:
         """False forces the plain thread-per-env step kernel (the TMA-staged kernel is the default where it applies)."""
         _native.check(self._lib.cavgym_set_step_path(self._handle, int(bool(use_tma))))
 
-    def set_rollout_path(self, team=True):
-        """True runs cavgym_rollout of a heterogeneous scenario of three or more bodies on the team-of-warps kernel
-        (kernels_team.cuh: one warp per body; bitwise the thread-per-env kernel, which stays the default)."""
-        _native.check(self._lib.cavgym_set_rollout_path(self._handle, int(bool(team))))
-
     def set_dense_path(self, force=True):
         """True runs a small scenario through the warp-per-env kernels that scenarios with > CAV_SMALL_M bodies always use."""
         _native.check(self._lib.cavgym_set_dense_path(self._handle, int(bool(force))))

@@ -238,9 +238,7 @@ typedef struct CavRolloutRecord {
 } CavRolloutRecord;
 
 /* cavgym_rollout that also writes `rec` (HOST struct of device pointers; NULL or all-NULL = cavgym_rollout).  The launches,
- * engine state, counters, episode-log rows and t_global afterwards are exactly those of cavgym_rollout.  With
- * cavgym_set_rollout_path(team = 1) a recorded rollout runs the thread-per-environment kernel (the team kernel forms no
- * rewards); its results are bitwise the same. */
+ * engine state, counters, episode-log rows and t_global afterwards are exactly those of cavgym_rollout. */
 int cavgym_rollout_record(CavEngine* engine, int n_steps, int auto_reset, const CavRolloutRecord* rec, cudaStream_t stream);
 
 /* Replayed joint actions, n_steps transitions in one launch:
@@ -357,13 +355,6 @@ int cavgym_set_action_logging(CavEngine* engine, int enabled);
  * aligned buffers) and the plain thread-per-env kernel for whatever is left; use_tma = 0 forces the plain kernel
  * everywhere (A/B measurements, parity of the two paths). */
 int cavgym_set_step_path(CavEngine* engine, int use_tma);
-
-/* cavgym_rollout of a heterogeneous scenario of 3..CAV_SMALL_M bodies (crossroads, bus stop, pelican crossing:
- * examples/environments/*.py) has a second implementation: a team of M warps per 32 environments, one warp per body, bodies
- * in registers and meeting through shared memory (kernels_team.cuh).  Results are bitwise those of the thread-per-environment
- * kernel; measured it is no faster (DESIGN 4.6), so it is opt-in: team = 1 selects it, 0 (default) goes back.  Scenarios of
- * the Pedestrians-v0 family, one- and two-body scenarios and election agents always run thread per environment. */
-int cavgym_set_rollout_path(CavEngine* engine, int team);
 
 /* Scenarios with more than CAV_SMALL_M bodies always run the warp-per-environment kernels (one env per warp, bodies
  * staged in shared memory, fp32 broad phase + exact narrow phase for the all-pairs collision test of

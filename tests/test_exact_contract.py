@@ -9,7 +9,7 @@ and useful only if the flag is not raised without a cause.  Here a placement gen
 (multiples of tau) from every decision boundary and on every branch of `road_share` (one kerb, kerb touch, road corner:
 axis-aligned shortcut, wedge, clipper, apart), each env of a batch one configuration stepped once with zero actions.  The
 exact truth (tests/exact_geometry.py, rational arithmetic) is computed on the post-step state the engine returns, and every
-kernel path (TMA / plain step, replay T = 1 and 3, warp-per-env, thread-per-env and team rollouts) must agree bitwise and
+kernel path (TMA / plain step, replay T = 1 and 3, warp-per-env, the thread-per-env rollout) must agree bitwise and
 meet, in fp64 and fp32:
   soundness    a decision that differs from the exact one is flagged;
   sensitivity  a consulted margin with |m| <= tau/2, or a share with |p - 0.5| <= tau/2, is flagged;
@@ -817,20 +817,17 @@ def run_paths(name, dtype):
             assert np.array_equal(a, b, equal_nan=True), f"{name}/{dtype}: {path} differs from step_tma in {key}"
     for key, a, b in zip(keys + ("liveness",), ref, stepped[0]):
         assert np.array_equal(a, b, equal_nan=True), f"{name}/{dtype}: the first of three steps differs from step_tma in {key}"
-    if cat.scenario in HETEROGENEOUS:   # thread-per-env and team rollouts with noop agents
-        for team in (False, True):
-            agents = make_env(compile_category(cat, "noop", dtype), n, dtype)
-            agents.set_rollout_path(team)
-            agents.reset(init_state=init)
-            agents.rollout(1, auto_reset=False)
-            torch.cuda.synchronize()
-            label = "team" if team else "thread-per-env"
-            assert np.array_equal(agents.state.cpu().numpy(), ref[0]), f"{name}/{dtype}: {label} rollout state"
-            assert np.array_equal(agents.episode_liveness.cpu().numpy(), ref[5]), f"{name}/{dtype}: {label} rollout liveness"
-            assert np.array_equal(agents.done_latch.cpu().numpy(), ref[2]), f"{name}/{dtype}: {label} rollout done"
-            assert np.array_equal(agents.winner_latch.cpu().numpy(), ref[3]), f"{name}/{dtype}: {label} rollout winner"
-            assert agents.stats()["tangent"] == int(ref[4].astype(bool).sum()), f"{name}/{dtype}: {label} rollout tangent count"
-            agents.close()
+    if cat.scenario in HETEROGENEOUS:   # thread-per-env rollout with noop agents
+        agents = make_env(compile_category(cat, "noop", dtype), n, dtype)
+        agents.reset(init_state=init)
+        agents.rollout(1, auto_reset=False)
+        torch.cuda.synchronize()
+        assert np.array_equal(agents.state.cpu().numpy(), ref[0]), f"{name}/{dtype}: thread-per-env rollout state"
+        assert np.array_equal(agents.episode_liveness.cpu().numpy(), ref[5]), f"{name}/{dtype}: thread-per-env rollout liveness"
+        assert np.array_equal(agents.done_latch.cpu().numpy(), ref[2]), f"{name}/{dtype}: thread-per-env rollout done"
+        assert np.array_equal(agents.winner_latch.cpu().numpy(), ref[3]), f"{name}/{dtype}: thread-per-env rollout winner"
+        assert agents.stats()["tangent"] == int(ref[4].astype(bool).sum()), f"{name}/{dtype}: thread-per-env rollout tangent count"
+        agents.close()
     return ref
 
 

@@ -33,7 +33,6 @@ CASES = {
     "election": ("learn_election3_seed22", 203, ()),
     "warp_per_env_forced": ("pedestrians_rc_eps05_seed1", 75, (("set_dense_path", True),)),
     "warp_per_env_320_bodies": ("dense320", 37, ()),
-    "team_falls_back": ("busstop_random_all_seed8", 203, (("set_rollout_path", True),)),
 }
 
 

@@ -86,8 +86,6 @@ CASES = {
                              {"state", "agent", "t_ep", "done", "winner", "active"}),
     "rollout_homogeneous": ("pedestrians_rc_eps05_seed1", "device", 1000, 500, (), "rollout", {"state", "cs", "agent", "t_ep", "episode"}),
     "rollout_heterogeneous": ("busstop_random_all_seed8", "device", 1000, 300, (), "rollout", {"state", "action", "t_ep", "episode"}),
-    "rollout_team": ("busstop_random_all_seed8", "device", 1000, 300, (("set_rollout_path", True),), "rollout",
-                     {"state", "action", "t_ep", "episode"}),
     "rollout_election": ("learn_election3_seed22", "device", 300, 300, (), "rollout", {"state", "agent", "t_ep", "episode", "active"}),
     "warp_per_env_forced": ("pedestrians_rc_eps05_seed1", "device", 300, 500, (("set_dense_path", True),), "rollout",
                             {"state", "cs", "agent", "t_ep", "episode"}),
