@@ -21,6 +21,7 @@
 #endif
 #include "kernels_tma.cuh"   // (tma_span, kReplayTile for the replay launch chain; includes kernels_small.cuh)
 #include "kernels_snapshot.cuh"
+#include "kernels_until.cuh"
 
 namespace cav {
 
@@ -29,7 +30,9 @@ namespace cav {
   extern const SmallLaunchers<double> kSmallF64M##K;     \
   extern const SmallLaunchers<float> kSmallF32M##K;      \
   extern const RolloutRecordLauncher<double> kRecordF64M##K; \
-  extern const RolloutRecordLauncher<float> kRecordF32M##K;
+  extern const RolloutRecordLauncher<float> kRecordF32M##K; \
+  extern const RolloutUntilLauncher<double> kUntilF64M##K; \
+  extern const RolloutUntilLauncher<float> kUntilF32M##K;
 CAV_FOR_EACH_M(CAV_DECLARE)
 #undef CAV_DECLARE
 
@@ -61,6 +64,23 @@ template <> RolloutRecordLauncher<double> rollout_record_launcher<double>(int m)
 template <> RolloutRecordLauncher<float> rollout_record_launcher<float>(int m) {
   switch (m) {
 #define CAV_CASE(K) case K: return kRecordF32M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+
+template <> RolloutUntilLauncher<double> rollout_until_launcher<double>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kUntilF64M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+template <> RolloutUntilLauncher<float> rollout_until_launcher<float>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kUntilF32M##K;
     CAV_FOR_EACH_M(CAV_CASE)
 #undef CAV_CASE
     default: return nullptr;
@@ -915,6 +935,30 @@ int cavgym_rollout_record(CavEngine* eng, int n_steps, int auto_reset, const Cav
   if (n_steps == 0) return CAV_OK;
   rc = eng->dtype == CAV_F64 ? rollout_record_typed(eng, eng->sc64, eng->buf64, *rec, n_steps, auto_reset, stream)
                              : rollout_record_typed(eng, eng->sc32, eng->buf32, *rec, n_steps, auto_reset, stream);
+  if (rc) return rc;
+  eng->t_global += n_steps;
+  return CAV_OK;
+}
+
+int cavgym_rollout_until(CavEngine* eng, int n_steps, double level, uint64_t salt, void* score, uint8_t* status, cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!score || !status) return fail(CAV_EINVAL, "score/status is NULL");
+  if (n_steps < 0) return fail(CAV_EINVAL, "n_steps must be >= 0");
+  if (std::isnan(level)) return fail(CAV_EINVAL, "level is NaN");
+  bool pedestrian = false;
+  for (int b = 1; b < eng->m; ++b) pedestrian = pedestrian || (eng->bodies[(size_t)b].flags & CAV_FLAG_PEDESTRIAN) != 0;
+  if (!eng->host.terminate_ego_zones || !pedestrian)
+    return fail(CAV_EINVAL, "no tester can win this scenario: cavgym_rollout_until needs terminate_ego_zones and a Pedestrian body");
+  if (eng->has_external) return fail(CAV_ESTATE, "cavgym_rollout_until needs an on-device agent for every body");
+  if (eng->dense) return fail(CAV_ESTATE, "cavgym_rollout_until runs on the thread-per-environment path only (at most CAV_SMALL_M bodies, "
+                                          "cavgym_set_dense_path off)");
+  if (n_steps == 0) return CAV_OK;
+  if (eng->dtype == CAV_F64)
+    rollout_until_launcher<double>(eng->m)(eng->sc64, eng->buf64, (double*)score, status, level, salt, eng->t_global, n_steps, stream);
+  else
+    rollout_until_launcher<float>(eng->m)(eng->sc32, eng->buf32, (float*)score, status, level, salt, eng->t_global, n_steps, stream);
+  rc = launch_check(eng, "rollout until kernel");
   if (rc) return rc;
   eng->t_global += n_steps;
   return CAV_OK;

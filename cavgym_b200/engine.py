@@ -212,6 +212,33 @@ class BatchedCAVEnv:
         _native.check(self._lib.cavgym_rollout_record(self._handle, n_steps, int(bool(auto_reset)), C.byref(rec), self._stream()))
         return out
 
+    @property
+    def max_timesteps(self):
+        """The scenario's episode length (config.json "max_timesteps")."""
+        return int(self.compiled.struct.max_timesteps)
+
+    UNTIL_LIVE, UNTIL_PARKED, UNTIL_FINISHED = 0, 1, 2
+
+    def rollout_until(self, n_steps, level, score, salt=0, status=None):
+        """rollout(n_steps, auto_reset=False) that parks each env at the first step where its score reaches `level`
+        (cavgym_rollout_until): score = running max of the danger (px by which a pedestrian overlaps the ego's reaction
+        zone), +inf once a tester wins.  `score` is the caller's contiguous [N] tensor of the engine's dtype on its device,
+        read and updated in place.  Returns `status` (uint8 [N], new unless given): UNTIL_LIVE, UNTIL_PARKED (tester wins
+        included) or UNTIL_FINISHED.  salt = 0 steps on the engine's random streams; another salt on fresh ones for this call
+        only (splitting.py forks envs between calls).  With n_steps = 0 nothing runs and `status` is left as it was."""
+        n = self.num_envs
+        if not (isinstance(score, torch.Tensor) and score.dtype == self.dtype and tuple(score.shape) == (n,)
+                and score.device == self.device and score.is_contiguous()):
+            raise ValueError(f"score must be a contiguous {self.dtype} tensor of shape ({n},) on {self.device}")
+        if status is None:
+            status = torch.zeros(n, dtype=torch.uint8, device=self.device)
+        elif not (isinstance(status, torch.Tensor) and status.dtype == torch.uint8 and tuple(status.shape) == (n,)
+                  and status.device == self.device and status.is_contiguous()):
+            raise ValueError(f"status must be a contiguous uint8 tensor of shape ({n},) on {self.device}")
+        _native.check(self._lib.cavgym_rollout_until(self._handle, int(n_steps), float(level), int(salt) % (1 << 64), _ptr(score),
+                                                     _ptr(status), self._stream()))
+        return status
+
     def replay(self, actions, record=("state", "reward", "done", "winner", "tangent")):
         """Replay joint actions [T,M,2,N] in one launch; returns the recorded trajectories as a dict."""
         n, m = self.num_envs, self.num_bodies

@@ -241,6 +241,31 @@ typedef struct CavRolloutRecord {
  * engine state, counters, episode-log rows and t_global afterwards are exactly those of cavgym_rollout. */
 int cavgym_rollout_record(CavEngine* engine, int n_steps, int auto_reset, const CavRolloutRecord* rec, cudaStream_t stream);
 
+/* One stage of a multilevel splitting estimate of the rate of "interesting" episodes, those a tester wins (winner > 0,
+ * reporting.py:227-243): Simulation.run's loop (simulation.py:38-118) as cavgym_rollout with auto_reset = 0, that also
+ * carries a caller-owned score per env and PARKS an env at the first step where its score reaches `level`.
+ *   danger of a post-step state: -min over the Pedestrian bodies of the separating-axis margin of the body's box against
+ *     the ego's reaction-zone rectangle (environment.py:195-206), in px, positive on overlap; the rectangle is taken whether
+ *     or not the zones exist (the ego steering, or standing still).
+ *   at entry: an env with done != 0 is not stepped: parked with score = +inf if its latched winner is > 0, finished
+ *     otherwise.  A live env with score >= level is parked without a step (so a repeated launch changes nothing, and a
+ *     launch at a higher level resumes it).
+ *   per step: a step that ends the episode with winner > 0 sets score = +inf (parked); one that ends it otherwise (done, or
+ *     cut off at max_timesteps) finishes the env and leaves its score; any other step sets score = max(score, danger) and
+ *     parks the env once score >= level.  A parked env keeps the state of that step, as a finished env is frozen.
+ * score   device real[N], read and written.  status  device u8[N]: 0 = live below the level after n_steps, 1 = parked
+ *         (tester wins included), 2 = finished without reaching the level.
+ * Every step taken is scored, logged and counted as cavgym_rollout's; t_global advances by n_steps.
+ * salt = 0 draws the engine's Philox streams bit for bit; any other salt keys this launch's draws with
+ * seed ^ splitmix64(salt) instead (the engine's seed, cavgym_save_engine included, is unchanged): the fresh randomness a
+ * copy made by cavgym_fork_envs needs, since its slot's own stream at the same (episode, t) drew the trajectory that was
+ * just discarded.  An ordinary launch on `stream`.  n_steps = 0 does nothing.
+ * CAV_EINVAL: NULL engine, score or status, n_steps < 0, NaN level, a scenario no tester can win (terminate_ego_zones off
+ * or no Pedestrian body).  CAV_ESTATE: a body with CAV_AGENT_EXTERNAL, or the warp-per-environment path (more than
+ * CAV_SMALL_M bodies, or cavgym_set_dense_path(1)). */
+int cavgym_rollout_until(CavEngine* engine, int n_steps, double level, uint64_t salt, void* score, uint8_t* status,
+                         cudaStream_t stream);
+
 /* Replayed joint actions, n_steps transitions in one launch:
  * actions real[T][M][2][N]; trajectory outputs (each nullable) state real[T][M][4][N],
  * reward real[T][M][N], done u8[T][N], winner i32[T][N], tangent u8[T][N].
