@@ -1,5 +1,6 @@
 """Shared test utilities: golden fixtures and scenario construction from their metadata."""
 import json
+import math
 import os
 from types import SimpleNamespace
 
@@ -123,3 +124,124 @@ def state_err_trajectory(got, want):
     d = got[..., 3] - want[..., 3]
     ang = np.abs(np.arctan2(np.sin(d), np.cos(d))) / np.maximum(1.0, np.abs(want[..., 3]))
     return float(max(pos.max(), vel.max(), ang.max()))
+
+
+# ------------------------------------------------------------------ the (body count, scenario family) matrix
+def random_actions(rng, t_len, n, is_car):
+    """Valid joint actions [T, M, 2, N]: cars brake / accelerate and steer a little, pedestrians wander."""
+    m = len(is_car)
+    car = np.asarray(is_car, dtype=bool)[None, :, None]
+    actions = np.zeros((t_len, m, 2, n))
+    hold = rng.random((t_len, m, n)) < 0.1
+    throttle = rng.uniform(-140.0, 140.0, (t_len, m, n))
+    steer_car = rng.uniform(-0.3, 0.3, (t_len, m, n))
+    steer_ped = rng.uniform(-0.4 * np.pi, 0.4 * np.pi, (t_len, m, n))
+    actions[:, :, 0] = np.where(hold & car, throttle, 0.0)
+    actions[:, :, 1] = np.where(car, np.where(hold, steer_car, 0.0), np.where(rng.random((t_len, m, n)) < 0.3, steer_ped, 0.0))
+    return actions
+
+
+def check_against_oracle(got, want, dtype):
+    """Trajectories [T, ...]: events identical off flagged steps; state / rewards compared up to the first flagged
+    divergence of each env."""
+    want_state, want_reward, want_done, want_winner, _ = want
+    tangent = got["tangent"].astype(bool)
+    mismatch = (got["done"] != want_done) | (got["winner"] != want_winner)
+    assert not np.any(mismatch & ~tangent), f"unflagged event mismatch at {np.argwhere(mismatch & ~tangent)[:5]}"
+    t_len, n = mismatch.shape
+    err = state_err if dtype == "float64" else state_err_trajectory
+    worst = 0.0
+    for e in range(n):
+        stop = int(np.nonzero(mismatch[:, e])[0][0]) if mismatch[:, e].any() else t_len
+        worst = max(worst, err(np.moveaxis(got["state"][:stop, :, :, e], 2, -1), np.moveaxis(want_state[:stop, :, :, e], 2, -1)))
+        assert rel_err(got["reward"][:stop, :, e], want_reward[:stop, :, e]) < (1e-9 if dtype == "float64" else 2e-3)
+    assert worst < (1e-9 if dtype == "float64" else 1e-4), worst
+    return int(want_done.any(axis=0).sum())
+
+
+def custom_road_frames(snap):
+    """(rear centre, orientation, length) of the roads of the custom-road scenario: the stock major road, one minor road
+    rotated by 30 degrees, and two minor roads turned off the vertical by the angle that moves their far corners 0.5 and 2
+    times `snap` (the axis snap, tau / 1000, engine.cu::convert) off their bounding box.  Every road is two lanes of 58.4 px."""
+    return [((0.0, 0.0), 0.0, 1584.0), ((300.0, 58.4), math.pi / 6, 400.0),
+            ((800.0, 58.4), math.pi / 2 + math.asin(0.5 * snap / 300.0), 300.0),
+            ((1200.0, -58.4), -math.pi / 2 + math.asin(2.0 * snap / 300.0), 300.0)]
+
+
+def custom_road_map(snap):
+    from cavgym_b200.library import geometry
+    from cavgym_b200.library.assets import Road, RoadConstants, RoadMap
+    roads = [Road(RoadConstants(length=length, num_outbound_lanes=1, num_inbound_lanes=1, lane_width=58.4,
+                                position=geometry.Point(*origin), orientation=phi)) for origin, phi, length in custom_road_frames(snap)]
+    return RoadMap(major_road=roads[0], minor_roads=roads[1:])
+
+
+MATRIX_M = tuple(range(1, 9))
+FAMILIES = ("homogeneous", "generic")
+TAU = {"float64": 1e-7, "float32": 5e-2}
+
+
+def matrix_scenario(m, family, mode, max_timesteps=60):
+    """One cell of the (body count, family) matrix of the thread-per-env kernels, M = 1..8.
+
+    homogeneous: Pedestrians-v0, the ego and m - 1 spawned pedestrians (every road an axis-aligned rectangle, every body
+                 after the ego a dynamic pedestrian: the GENERIC = false instantiations);
+    generic:     the custom road map (the same major road, and minor roads that are not axis-aligned: one rotated by 30
+                 degrees, two skewed off the vertical) with, for m >= 2, body 1 an oncoming car in the inbound lane, then
+                 m - 2 pedestrians.  The car alone already makes the scenario generic, but the GENERIC = false kernels give
+                 the same answers for it; bodies on the rotated roads are what only the generic kernels get right.
+    mode 'external' replays joint actions; 'device' drives the ego with a noop agent (a RandomAgent when it is alone, so
+    that envs differ), the car with a RandomAgent and the pedestrians with RandomConstrained agents.  `is_car` marks the
+    bodies that take car actions."""
+    from cavgym_b200.examples.environments import pedestrians as mod
+    from cavgym_b200.examples.constants import car_constants
+    from cavgym_b200.library.bodies import Car, DynamicBodyState
+    assert m in MATRIX_M and family in FAMILIES
+    constants = mod.env_constants
+    car = family == "generic" and m >= 2
+    bodies = mod.make_bodies(m - 1 - car, 1.0, 1.0, np_random=np.random.RandomState(0))
+    if car:
+        lane = mod.major_road.inbound.lanes[0]
+        bodies.insert(1, Car(DynamicBodyState(lane.spawn, car_constants.max_velocity / 2, mod.major_road.inbound.orientation),
+                             car_constants))
+    if family == "generic":
+        constants = SimpleNamespace(viewer_width=mod.env_constants.viewer_width, road_map=custom_road_map(TAU["float64"] * 1e-3))
+    is_car = np.array([b == 0 or (car and b == 1) for b in range(m)])
+    if mode == "external":
+        specs = [AgentSpec("external") for _ in bodies]
+    else:
+        specs = [AgentSpec("random", epsilon=0.05) if m == 1 else AgentSpec("noop")]
+        specs += [AgentSpec("random", epsilon=0.05) if is_car[b] else AgentSpec("random-constrained", epsilon=0.5) for b in range(1, m)]
+    config = SimpleNamespace(terminate_collisions="ego", terminate_ego_zones=True, terminate_ego_offroad=False,
+                             max_timesteps=max_timesteps, reward_win=6000.0, reward_draw=2000.0, cost_step=4.0)
+    comp = compile_scenario(bodies, constants, config, specs)
+    comp.is_car = is_car
+    return comp
+
+
+def expect_homogeneous(compiled, dtype="float64"):
+    """engine.cu::convert's rule, restated on the compiled tables: at most CAV_SMALL_M bodies, every road an axis-aligned
+    rectangle (every corner within tau / 1000 of its bounding box, in the engine's precision), every body dynamic and every
+    body after the ego a pedestrian."""
+    from cavgym_b200 import _abi
+    s = compiled.struct
+    if s.n_bodies > _abi.CAV_SMALL_M:
+        return False
+    to = np.float64 if dtype == "float64" else np.float32
+    snap = float(to(TAU[dtype] * 1e-3))
+    for r in range(s.n_roads):
+        xs = [float(to(s.roads[r].x[i])) for i in range(4)]
+        ys = [float(to(s.roads[r].y[i])) for i in range(4)]
+        for vs in (xs, ys):
+            lo, hi = min(vs), max(vs)
+            if any(min(abs(v - lo), abs(v - hi)) > snap for v in vs) or not hi > lo:
+                return False
+    for b in range(s.n_bodies):
+        if s.bodies[b].kind != _abi.CAV_BODY_DYNAMIC or (b > 0 and not s.bodies[b].flags & _abi.CAV_FLAG_PEDESTRIAN):
+            return False
+    return True
+
+
+def has_pedestrian(m, family):
+    """Whether the matrix cell (m, family) holds a pedestrian (the danger of the parking rollout needs one)."""
+    return m - 1 - (family == "generic" and m >= 2) > 0

@@ -26,7 +26,7 @@ import numpy as np
 import pytest
 
 import exact_geometry as xg
-from helpers import GOLDEN_DIR
+from helpers import GOLDEN_DIR, custom_road_frames, custom_road_map
 from cavgym_b200 import _abi
 
 TAU = {"float64": 1e-7, "float32": 5e-2}
@@ -57,24 +57,6 @@ class QuadObstacle:
 OBSTACLE = [(560.0, 20.0), (645.0, 34.0), (652.0, -27.0), (571.0, -41.0)]
 
 
-def custom_road_frames(dtype):
-    """(rear centre, orientation, length) of the roads of the custom-road scenario: the stock major road, one minor road
-    rotated by 30 degrees, and two minor roads turned off the vertical by the angle that moves their far corners 0.5 and 2
-    times the axis snap (tau / 1000, engine.cu::convert) off their bounding box.  Every road is two lanes of 58.4 px."""
-    snap = TAU[dtype] * 1e-3
-    return [((0.0, 0.0), 0.0, 1584.0), ((300.0, 58.4), math.pi / 6, 400.0),
-            ((800.0, 58.4), math.pi / 2 + math.asin(0.5 * snap / 300.0), 300.0),
-            ((1200.0, -58.4), -math.pi / 2 + math.asin(2.0 * snap / 300.0), 300.0)]
-
-
-def custom_road_map(dtype):
-    from cavgym_b200.library import geometry
-    from cavgym_b200.library.assets import Road, RoadConstants, RoadMap
-    roads = [Road(RoadConstants(length=length, num_outbound_lanes=1, num_inbound_lanes=1, lane_width=58.4,
-                                position=geometry.Point(*origin), orientation=phi)) for origin, phi, length in custom_road_frames(dtype)]
-    return RoadMap(major_road=roads[0], minor_roads=roads[1:])
-
-
 def compile_category(cat, agents, dtype="float64"):
     from cavgym_b200.scenario import AgentSpec, compile_scenario
     if cat.scenario in ("pedestrians", "obstacle", "custom-roads"):
@@ -96,7 +78,7 @@ def compile_category(cat, agents, dtype="float64"):
         road_map.set_obstacle(QuadObstacle(OBSTACLE))
         constants = SimpleNamespace(viewer_width=mod.env_constants.viewer_width, road_map=road_map)
     elif cat.scenario == "custom-roads":
-        constants = SimpleNamespace(viewer_width=mod.env_constants.viewer_width, road_map=custom_road_map(dtype))
+        constants = SimpleNamespace(viewer_width=mod.env_constants.viewer_width, road_map=custom_road_map(TAU[dtype] * 1e-3))
     specs = [AgentSpec(agents) for _ in bodies]
     return compile_scenario(bodies, constants, env_config(cat.collisions, cat.offroad), specs)
 
@@ -525,7 +507,7 @@ def in_frame(state, origin, phi):
 def gen_custom_roads(desc, tau, rng, dtype="float64"):
     """Pedestrians across the kerbs and far corners of the rotated road and of the two roads on either side of the axis
     snap; the ego at k tau from their edges, off the major road (off-road against a rotated road)."""
-    frames = custom_road_frames(dtype)
+    frames = custom_road_frames(TAU[dtype] * 1e-3)
     out = []
     for b in range(3):
         r = int(rng.integers(1, 4))

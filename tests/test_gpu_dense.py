@@ -11,7 +11,7 @@ from types import SimpleNamespace
 import numpy as np
 import pytest
 
-from helpers import compile_from_meta, load_golden, rel_err, soa, state_err, state_err_trajectory
+from helpers import check_against_oracle, compile_from_meta, load_golden, random_actions, soa, state_err
 
 pytestmark = pytest.mark.gpu
 
@@ -36,20 +36,6 @@ def dense_scenario(mode, num_cars=64, num_pedestrians=256, epsilon=0.002, collis
     comp = compile_scenario(bodies, constants, dense_config(collisions), specs)
     comp.is_car = np.array([not isinstance(body, Pedestrian) for body in bodies])
     return comp
-
-
-def random_actions(rng, t_len, n, is_car):
-    """Valid joint actions [T, M, 2, N]: cars brake / accelerate and steer a little, pedestrians wander."""
-    m = len(is_car)
-    car = is_car[None, :, None]
-    actions = np.zeros((t_len, m, 2, n))
-    hold = rng.random((t_len, m, n)) < 0.1
-    throttle = rng.uniform(-140.0, 140.0, (t_len, m, n))
-    steer_car = rng.uniform(-0.3, 0.3, (t_len, m, n))
-    steer_ped = rng.uniform(-0.4 * np.pi, 0.4 * np.pi, (t_len, m, n))
-    actions[:, :, 0] = np.where(hold & car, throttle, 0.0)
-    actions[:, :, 1] = np.where(car, np.where(hold, steer_car, 0.0), np.where(rng.random((t_len, m, n)) < 0.3, steer_ped, 0.0))
-    return actions
 
 
 def make(comp, n, dtype, **kw):
@@ -146,24 +132,6 @@ def test_rollout_without_auto_reset_on_a_ragged_batch(name):
 
 
 # ------------------------------------------------------------------ dense traffic (C4) vs the oracle
-def check_against_oracle(got, want, dtype):
-    """Trajectories [T, ...]: events identical off flagged steps; state / rewards compared up to the first flagged
-    divergence of each env."""
-    want_state, want_reward, want_done, want_winner, _ = want
-    tangent = got["tangent"].astype(bool)
-    mismatch = (got["done"] != want_done) | (got["winner"] != want_winner)
-    assert not np.any(mismatch & ~tangent), f"unflagged event mismatch at {np.argwhere(mismatch & ~tangent)[:5]}"
-    t_len, n = mismatch.shape
-    err = state_err if dtype == "float64" else state_err_trajectory
-    worst = 0.0
-    for e in range(n):
-        stop = int(np.nonzero(mismatch[:, e])[0][0]) if mismatch[:, e].any() else t_len
-        worst = max(worst, err(np.moveaxis(got["state"][:stop, :, :, e], 2, -1), np.moveaxis(want_state[:stop, :, :, e], 2, -1)))
-        assert rel_err(got["reward"][:stop, :, e], want_reward[:stop, :, e]) < (1e-9 if dtype == "float64" else 2e-3)
-    assert worst < (1e-9 if dtype == "float64" else 1e-4), worst
-    return int(want_done.any(axis=0).sum())
-
-
 @pytest.mark.parametrize("dtype", ["float64", "float32"])
 def test_dense_traffic_replay_matches_oracle(dtype):
     """64 cars + 256 pedestrians, random valid joint actions: cavgym_replay and cavgym_step vs the oracle."""
@@ -395,3 +363,98 @@ def test_six_and_eight_body_scenarios_replay_and_step(pedestrians, dtype):
         oracle.reset(init_state=init)
         want = oracle.replay(actions[:steps // 2])
         check_against_oracle({k: v for k, v in outs[0][0].items()}, want, dtype)
+
+
+# ------------------------------------------------------------------ the pair sweep at every tile shape, planted pairs
+# kernels_dense.cuh pads M to Mp = (M + 31) & ~31 and sweeps pairs in passes of two 32-body tiles; these body counts give a
+# ragged or full last tile, an odd or even tile count, and a final pass of one tile with tiles below it (65..96, 129..160)
+SWEEP_M = (9, 31, 32, 33, 63, 64, 65, 96, 97, 128, 129, 160, 161, 320, 511, 512)
+SPACING = 400.0     # lattice pitch: more than twice the sum of the largest half-diagonals (a car: 38.6 px) plus both lengths
+
+
+def planted_pairs(m):
+    """(i, j), i < j: every unordered pair up to 161 bodies; above, every within-tile offset 1..31 in every tile and every
+    pair of tiles at three lane pairs (the lower tile against tile A and tile B of each pass)."""
+    if m <= 161:
+        i, j = np.triu_indices(m, 1)
+        return np.stack([i, j], axis=1)
+    tiles = (m + 31) // 32
+    pairs = [(32 * t + (t * 5 + 3 * d) % (32 - d), 32 * t + (t * 5 + 3 * d) % (32 - d) + d) for t in range(tiles) for d in range(1, 32)]
+    pairs += [(32 * a + la, 32 * b + lb) for a in range(tiles) for b in range(a + 1, tiles) for la, lb in ((0, 31), (31, 0), (13, 6))]
+    return np.array([p for p in pairs if p[1] < m])
+
+
+def planted_batch(comp, pairs, shuffled, x0, depth, rng):
+    """Initial states [M, 4, N] of one env per pair plus 8 controls: the ego parked at (100, 0) heading along the road with
+    v = 0 (no stopping zones), every other body still on a lattice of pitch SPACING from (x0, 3000) — in body order, or
+    shuffled so that every tile's union box spans the lattice — at a random heading; then body j of the env's pair moved
+    to overlap body i by `depth` px along i's axis, at i's heading (separating-axis margin -depth)."""
+    m = comp.n_bodies
+    types = comp.struct.types
+    hl = np.array([types[comp.struct.bodies[b].type_id].length / 2 for b in range(m)])
+    site = rng.permutation(m - 1) if shuffled else np.arange(m - 1)
+    n = len(pairs) + 8
+    state = np.zeros((m, 4, n))
+    state[1:, 0] = (x0 + SPACING * (site % 40))[:, None]
+    state[1:, 1] = (3000.0 + SPACING * (site // 40))[:, None]
+    state[1:, 3] = rng.uniform(-np.pi, np.pi, m - 1)[:, None]
+    state[0, 0] = 100.0
+    e = np.arange(len(pairs))
+    i, j = pairs[:, 0], pairs[:, 1]
+    th = state[i, 3, e]
+    reach = hl[i] + hl[j] - depth
+    state[j, 0, e] = state[i, 0, e] + reach * np.cos(th)
+    state[j, 1, e] = state[i, 1, e] + reach * np.sin(th)
+    state[j, 3, e] = th
+    return state
+
+
+@pytest.mark.parametrize("dtype", ["float64", "float32"])
+@pytest.mark.parametrize("m", SWEEP_M)
+def test_pair_sweep_finds_every_planted_pair(m, dtype):
+    """Exactly one overlapping (or nearly touching) pair per env, every pair of bodies (or, from 320 bodies, every within-tile
+    offset and every pair of tiles), the bodies in lattice order and shuffled, at depths -2 px, +-10 tau, and +-10 tau with
+    the lattice translated to x = 2e4 px (one float32 ulp ~ 2e-3 px: an fp64 pair 1e-6 px deep must pass the float32 broad
+    phase).  Every planted margin is more than 2 tau from 0, so `done` must be its exact decision and no env may be
+    flagged; the 8 control envs of each batch, with no planted pair, must not end.  Noop actions, velocity 0."""
+    import torch
+    import exact_geometry as xg
+    tau = {"float64": 1e-7, "float32": 5e-2}[dtype]
+    cars = max(1, m // 5)
+    comp = dense_scenario("external", num_cars=cars, num_pedestrians=m - cars)
+    assert comp.n_bodies == m
+    pairs = planted_pairs(m)
+    rng = np.random.default_rng(m)
+    batches, want = [], []
+    for x0, depth in ((400.0, 2.0), (400.0, 10 * tau), (400.0, -10 * tau), (2e4, 10 * tau), (2e4, -10 * tau)):
+        for shuffled in (False, True):
+            batches.append(planted_batch(comp, pairs, shuffled, x0, depth, rng))
+            want.append(np.concatenate([np.full(len(pairs), depth > 0), np.zeros(8, dtype=bool)]))
+    init, want = np.concatenate(batches, axis=-1), np.concatenate(want)
+    n = init.shape[-1]
+    env = make(comp, n, dtype, seed=4)
+    env.reset(init_state=init)
+    state, _, done, _, tangent = env.step(torch.zeros((m, 2, n), dtype=env.dtype, device=env.device))
+    done, tangent, state = done.cpu().numpy() != 0, tangent.cpu().numpy(), state.double().cpu().numpy()
+    assert not tangent.any(), f"flagged without a margin within 2 tau: envs {np.flatnonzero(tangent)[:5]}"
+    wrong = np.flatnonzero(done != want)
+    if wrong.size:
+        e = wrong[0] % (len(pairs) + 8)
+        pytest.fail(f"{wrong.size} envs wrong, first {wrong[0]}: pair {tuple(pairs[e]) if e < len(pairs) else 'control'}, "
+                    f"done {done[wrong[0]]}")
+    # the construction against exact arithmetic on the stepped state, on a sample of planted envs of every batch
+    types = comp.struct.types
+    dims = [(types[comp.struct.bodies[b].type_id].length, types[comp.struct.bodies[b].type_id].width) for b in range(m)]
+    per = len(pairs) + 8
+    for b in range(len(batches)):
+        for e in rng.choice(len(pairs), size=min(8, len(pairs)), replace=False):
+            i, j = pairs[e]
+            box = [xg.make_box(*dims[k], state[k, 3, b * per + e], state[k, 0, b * per + e], state[k, 1, b * per + e]) for k in (i, j)]
+            margin = xg.sat_margin(*box)
+            assert margin.cmp(0) == (-1 if want[b * per + e] else 1) and not margin.within(2 * tau), (b, i, j, float(margin))
+    # the lattice: in a control env no two bodies come within reach of each other
+    half_l = torch.tensor([d[0] / 2 for d in dims], dtype=torch.float64)
+    half_w = torch.tensor([d[1] / 2 for d in dims], dtype=torch.float64)
+    controls = [b * per + per - 1 for b in range(len(batches))]
+    hit, closest = all_pairs_reference(torch.tensor(state[:, :, controls]), half_l, half_w, torch.ones(m, dtype=torch.bool))
+    assert not hit.any() and float(closest.min()) > 100.0

@@ -20,7 +20,8 @@ events agree and ends at the first event difference (after it the two runs are d
 import numpy as np
 import pytest
 
-from helpers import GOLDEN_CASES, LEARN_CASES, compile_from_meta, load_golden, rel_err, soa, state_err, state_err_trajectory
+from helpers import (FAMILIES, GOLDEN_CASES, LEARN_CASES, MATRIX_M, compile_from_meta, load_golden, matrix_scenario, random_actions,
+                     rel_err, soa, state_err, state_err_trajectory)
 
 pytestmark = pytest.mark.gpu
 
@@ -380,25 +381,21 @@ def test_sharded_engines_match_one_engine(dtype):
     assert total == want and want["episodes"] > n
 
 
-def test_float32_wire_format_is_the_fp64_engine_on_widened_actions():
-    """cavgym_step_host_f32: float32 actions in, float32 state / rewards out, fp64 engine.  Against a second fp64 engine stepped
-    on the device with the widened actions: the engine states are BITWISE equal, the outputs are their float32 roundings, the
-    events identical."""
+def check_wire_format(compiled, init, actions):
+    """cavgym_step_host_f32 on `actions` [T, M, 2, N] nudged off float32-representable values, against a second fp64 engine
+    stepped on the device with the widened actions: the engine states are BITWISE equal, the outputs are their float32
+    roundings, the events identical.  `compiled`: two CompiledScenario of the same scenario; `init`: initial states or None
+    (both engines draw the same spawns).  Returns the wire engine's stats()."""
     import torch
-    meta, episodes = load_golden("learn_election3_seed22")      # four bodies; episodes of 116, 901, 218 and 79 steps
-    k, n, steps = len(episodes), 4096, 250
-    init = soa(np.stack([episodes[e % k]["init_state"] for e in range(n)]))
-    actions = np.zeros((steps, meta["n_bodies"], 2, n))
-    for j, ep in enumerate(episodes):
-        a = ep["actions"][:steps]
-        actions[:a.shape[0], :, :, j::k] = a[..., None]
-    actions *= 1.0 - 1e-4 * np.random.RandomState(0).uniform(0.1, 1.0, actions.shape)   # inside the bounds, not float32-representable
+    from cavgym_b200 import BatchedCAVEnv
+    steps, m, _, n = actions.shape
+    actions = actions * (1.0 - 1e-4 * np.random.RandomState(0).uniform(0.1, 1.0, actions.shape))   # inside the bounds
     wire = torch.tensor(actions, dtype=torch.float32).pin_memory()
-    a, b = make_env(meta, n, "float64"), make_env(meta, n, "float64")
+    a, b = (BatchedCAVEnv(None, None, None, num_envs=n, dtype="float64", compiled=c) for c in compiled)
     a.reset(init_state=init)
     b.reset(init_state=init)
-    h_state = torch.empty((meta["n_bodies"], 4, n), dtype=torch.float32).pin_memory()
-    h_reward = torch.empty((meta["n_bodies"], n), dtype=torch.float32).pin_memory()
+    h_state = torch.empty((m, 4, n), dtype=torch.float32).pin_memory()
+    h_reward = torch.empty((m, n), dtype=torch.float32).pin_memory()
     h_done, h_winner = torch.empty(n, dtype=torch.uint8).pin_memory(), torch.empty(n, dtype=torch.int32).pin_memory()
     h_tangent = torch.empty(n, dtype=torch.uint8).pin_memory()
     for t in range(steps):
@@ -407,9 +404,36 @@ def test_float32_wire_format_is_the_fp64_engine_on_widened_actions():
         assert torch.equal(a.state, b.state), t
         assert torch.equal(h_state, state.float().cpu()) and torch.equal(h_reward, reward.float().cpu()), t
         assert torch.equal(h_done, done.cpu()) and torch.equal(h_winner, winner.cpu()) and torch.equal(h_tangent, tangent.cpu()), t
-    assert a.stats() == b.stats() and a.stats()["episodes"] > n // 2 and a.stats()["errors"] == 0
+    assert a.stats() == b.stats() and a.stats()["errors"] == 0
     with pytest.raises(Exception, match="page-locked"):
         a.step_host(wire[0].clone(), h_state, h_reward, h_done, h_winner, h_tangent)      # pageable actions
+    return a.stats()
+
+
+def test_float32_wire_format_is_the_fp64_engine_on_widened_actions():
+    """cavgym_step_host_f32: float32 actions in, float32 state / rewards out, fp64 engine.  Against a second fp64 engine stepped
+    on the device with the widened actions: the engine states are BITWISE equal, the outputs are their float32 roundings, the
+    events identical."""
+    meta, episodes = load_golden("learn_election3_seed22")      # four bodies; episodes of 116, 901, 218 and 79 steps
+    k, n, steps = len(episodes), 4096, 250
+    init = soa(np.stack([episodes[e % k]["init_state"] for e in range(n)]))
+    actions = np.zeros((steps, meta["n_bodies"], 2, n))
+    for j, ep in enumerate(episodes):
+        a = ep["actions"][:steps]
+        actions[:a.shape[0], :, :, j::k] = a[..., None]
+    stats = check_wire_format([compile_from_meta(meta) for _ in range(2)], init, actions)
+    assert stats["episodes"] > n // 2
+
+
+@pytest.mark.parametrize("m, family", [pytest.param(m, family, id=f"{family}_m{m}") for family in FAMILIES for m in MATRIX_M])
+def test_float32_wire_format_in_every_body_count_and_family(m, family):
+    """The same on random valid actions in every (body count, family) cell of helpers.matrix_scenario, so that each
+    instantiation of step_wire32_kernel runs: 692 envs, max_timesteps 60, every env times out inside the 90 steps."""
+    n, steps = 692, 90
+    compiled = [matrix_scenario(m, family, "external", max_timesteps=60) for _ in range(2)]
+    actions = random_actions(np.random.RandomState(m), steps, n, compiled[0].is_car)
+    stats = check_wire_format(compiled, None, actions)
+    assert stats["episodes"] >= n
 
 
 def test_sweep_totals_do_not_depend_on_the_split():

@@ -14,7 +14,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import compile_from_meta, load_golden, state_err
+from helpers import compile_from_meta, load_golden, matrix_scenario, state_err
 
 pytestmark = pytest.mark.gpu
 
@@ -34,9 +34,15 @@ CASES = {
     "warp_per_env_forced": ("pedestrians_rc_eps05_seed1", 75, (("set_dense_path", True),)),
     "warp_per_env_320_bodies": ("dense320", 37, ()),
 }
+# the other cells of the (body count, family) matrix of helpers.matrix_scenario: every M = 1..8 of both families runs here
+MATRIX_CELLS = [(1, "homogeneous"), (3, "homogeneous"), (5, "homogeneous"), (6, "homogeneous"), (7, "homogeneous"),
+                (8, "homogeneous"), (1, "generic"), (2, "generic"), (4, "generic"), (6, "generic"), (7, "generic"), (8, "generic")]
+CASES.update({f"matrix_{family}_{m}_bodies": (("matrix", m, family), 203, ()) for m, family in MATRIX_CELLS})
 
 
 def compiled(name, mode):
+    if isinstance(name, tuple):
+        return matrix_scenario(name[1], name[2], mode, max_timesteps=MAX_T)
     if name == "dense320":
         from cavgym_b200.examples.environments import dense_traffic
         from cavgym_b200.library.bodies import Pedestrian
@@ -173,7 +179,7 @@ def test_complete_episodes_replay_bitwise_on_external_actions(case, dtype, auto_
 
 # the C oracle has no election agents; the warp-per-env cases are held to the thread-per-env rows by the tests above
 ORACLE_CASES = ("homogeneous_2_bodies", "homogeneous_rolled_4_bodies", "synced_crossroads", "synced_bus_stop",
-                "synced_pelican_crossing")
+                "synced_pelican_crossing") + tuple(f"matrix_{family}_{m}_bodies" for m, family in MATRIX_CELLS)
 
 
 @pytest.mark.parametrize("auto_reset", [True, False], ids=["auto_reset", "no_reset"])

@@ -15,7 +15,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import compile_from_meta, load_golden
+from helpers import compile_from_meta, has_pedestrian, load_golden, matrix_scenario
 
 pytestmark = pytest.mark.gpu
 
@@ -29,10 +29,17 @@ CASES = {
     "pelican_crossing": "pelican_random_all_seed10",
     "election": "learn_election3_seed22",
 }
+# the cells of helpers.matrix_scenario that the recorded-rollout tests add, except those without a pedestrian (refused below)
+MATRIX_CELLS = [(1, "homogeneous"), (3, "homogeneous"), (5, "homogeneous"), (6, "homogeneous"), (7, "homogeneous"),
+                (8, "homogeneous"), (1, "generic"), (2, "generic"), (4, "generic"), (6, "generic"), (7, "generic"), (8, "generic")]
+CASES.update({f"matrix_{family}_{m}_bodies": ("matrix", m, family) for m, family in MATRIX_CELLS if has_pedestrian(m, family)})
 LIVE, PARKED, FINISHED = 0, 1, 2
 
 
 def compiled(golden, mode="device", **config):
+    if isinstance(golden, tuple):
+        assert not config
+        return matrix_scenario(golden[1], golden[2], mode, max_timesteps=MAX_T)
     meta = copy.deepcopy(load_golden(golden)[0])
     meta["config"]["max_timesteps"] = MAX_T
     meta["config"].update(config)
@@ -231,6 +238,7 @@ def test_refusals_come_before_any_launch():
              (engine("homogeneous_2_bodies"), {"level": math.nan}, EINVAL, None),
              (engine("homogeneous_2_bodies", terminate_ego_zones=False), {}, EINVAL, None),
              (engine("busstop_random_all_seed8"), {}, EINVAL, None),   # no Pedestrian body
+             *[(engine(("matrix", m, family)), {}, EINVAL, None) for m, family in MATRIX_CELLS if not has_pedestrian(m, family)],
              (engine("homogeneous_2_bodies", mode="external"), {}, ESTATE, None),
              (forced, {}, ESTATE, None), (dense320(), {}, ESTATE, None)]
     for env, args, code, null in cases:
