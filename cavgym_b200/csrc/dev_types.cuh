@@ -153,6 +153,14 @@ struct RolloutRecord {
   int32_t* timestep;   // [T][N] t_ep after step t, 0 where the env did not step
 };
 
+// cavgym_set_agent_params: per-env tester parameters, [M][N] with the env index fastest, each nullable (null = the scenario's
+// DevBody value).  Given by value to the parameter kernels only (kernels_params.cuh), for the reason RolloutRecord is.
+template <typename R>
+struct AgentParams {
+  const double* epsilon;   // RandomAgent / RandomConstrainedAgent epsilon, double in both modes as DevBody::epsilon
+  const R* threshold;      // ProximityAgent / ElectionAgent distance threshold
+};
+
 // cavgym_step_host_f32: joint actions and results cross the host link as float32 while the engine steps in its own type.
 struct WireIO32 {
   const float* actions;  // [M][2][N]

@@ -22,6 +22,7 @@
 #include "kernels_tma.cuh"   // (tma_span, kReplayTile for the replay launch chain; includes kernels_small.cuh)
 #include "kernels_snapshot.cuh"
 #include "kernels_until.cuh"
+#include "kernels_params.cuh"
 
 namespace cav {
 
@@ -32,7 +33,9 @@ namespace cav {
   extern const RolloutRecordLauncher<double> kRecordF64M##K; \
   extern const RolloutRecordLauncher<float> kRecordF32M##K; \
   extern const RolloutUntilLauncher<double> kUntilF64M##K; \
-  extern const RolloutUntilLauncher<float> kUntilF32M##K;
+  extern const RolloutUntilLauncher<float> kUntilF32M##K; \
+  extern const ParamsLaunchers<double> kParamsF64M##K; \
+  extern const ParamsLaunchers<float> kParamsF32M##K;
 CAV_FOR_EACH_M(CAV_DECLARE)
 #undef CAV_DECLARE
 
@@ -81,6 +84,23 @@ template <> RolloutUntilLauncher<double> rollout_until_launcher<double>(int m) {
 template <> RolloutUntilLauncher<float> rollout_until_launcher<float>(int m) {
   switch (m) {
 #define CAV_CASE(K) case K: return kUntilF32M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+
+template <> const ParamsLaunchers<double>* params_launchers<double>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return &kParamsF64M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+template <> const ParamsLaunchers<float>* params_launchers<float>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return &kParamsF32M##K;
     CAV_FOR_EACH_M(CAV_CASE)
 #undef CAV_CASE
     default: return nullptr;
@@ -491,7 +511,13 @@ struct CavEngine {
   uint64_t fingerprint = 0;      // of the scenario tables' contents (scenario_fingerprint)
   void* d_stage = nullptr;       // cavgym_fork_envs: snapshot of the sources, grown on demand, freed by cavgym_destroy
   size_t stage_bytes = 0;
+  // cavgym_set_agent_params: per-env tester parameters [m][n] (epsilon double, threshold real), allocated on first use
+  double* d_epsilon = nullptr;
+  void* d_threshold = nullptr;
+  unsigned int* d_param_flags = nullptr;
+  bool epsilon_set = false, threshold_set = false;
 
+  bool agent_params_set() const { return epsilon_set || threshold_set; }
   size_t real_size() const { return dtype == CAV_F64 ? 8 : 4; }
 };
 
@@ -575,6 +601,19 @@ static int launch_check(CavEngine* eng, const char* what, int n_launches = 1) {
   return CAV_OK;
 }
 
+template <typename R>
+static AgentParams<R> agent_params(const CavEngine* eng) {
+  return {eng->epsilon_set ? eng->d_epsilon : nullptr, eng->threshold_set ? (const R*)eng->d_threshold : nullptr};
+}
+
+// Per-env tester parameters are honoured by the thread-per-env step, rollout and recording kernels only.
+static int refuse_dense_with_params(CavEngine* eng, const char* what) {
+  if (eng->dense && eng->agent_params_set())
+    return fail(CAV_ESTATE, std::string(what) + ": per-env agent parameters are set (cavgym_set_agent_params) and the warp-per-env "
+                            "kernels do not read them; clear them or turn cavgym_set_dense_path off");
+  return CAV_OK;
+}
+
 static int do_reset(CavEngine* eng, const uint8_t* mask, const void* init, int first_time, cudaStream_t stream) {
   if (eng->dense) {
     if (eng->dtype == CAV_F64) dense_launchers<double>()->reset(eng->sc64, eng->tb64, eng->buf64, mask, (const double*)init, first_time, stream);
@@ -601,6 +640,10 @@ static int dense_run(CavEngine* eng, const DevScenario<R>& sc, const EnvBuffers<
 template <typename R>
 static int step_range_typed(CavEngine* eng, const DevScenario<R>& sc, EnvBuffers<R> buf, const StepIO<R>& io, cudaStream_t stream) {
   if (eng->dense) return dense_run(eng, sc, buf, io, 1, 0, 0, stream);
+  if (eng->has_device_agents && eng->agent_params_set()) {
+    params_launchers<R>(eng->m)->step(sc, buf, io, agent_params<R>(eng), eng->t_global, stream);
+    return launch_check(eng, "step kernel (agent parameters)");
+  }
   const SmallLaunchers<R>* k = small_launchers<R>(eng->m);
   int launches = 0;
   if (!eng->has_device_agents && eng->use_tma) {   // replayed actions: persistent TMA-staged kernel over the whole tiles
@@ -745,6 +788,10 @@ static int rollout_record_typed(CavEngine* eng, const DevScenario<R>& sc, const 
     if (!dense_launchers<R>()->rollout_record(sc, dense_tables<R>(eng), buf, rec, eng->t_global, n_steps, auto_reset, stream))
       return fail(CAV_ECUDA, "dense kernel set-up failed (shared memory opt-in)");
     return launch_check(eng, "dense record kernel");
+  }
+  if (eng->agent_params_set()) {
+    params_launchers<R>(eng->m)->rollout_record(sc, buf, rec, agent_params<R>(eng), eng->t_global, n_steps, auto_reset, stream);
+    return launch_check(eng, "rollout record kernel (agent parameters)");
   }
   rollout_record_launcher<R>(eng->m)(sc, buf, rec, eng->t_global, n_steps, auto_reset, stream);
   return launch_check(eng, "rollout record kernel");
@@ -896,6 +943,7 @@ int cavgym_step(CavEngine* eng, const void* actions, void* state_out, void* rewa
   int rc = check_engine(eng);
   if (rc) return rc;
   if (!actions && eng->has_external) return fail(CAV_EINVAL, "actions is NULL but a body has CAV_AGENT_EXTERNAL");
+  if ((rc = refuse_dense_with_params(eng, "cavgym_step"))) return rc;
   rc = step_range(eng, 0, eng->n, actions, state_out, reward_out, done_out, winner_out, tangent_flag_out, stream);
   if (rc) return rc;
   eng->t_global += 1;
@@ -907,6 +955,7 @@ int cavgym_rollout(CavEngine* eng, int n_steps, int auto_reset, cudaStream_t str
   if (rc) return rc;
   if (n_steps < 0) return fail(CAV_EINVAL, "n_steps must be >= 0");
   if (eng->has_external) return fail(CAV_ESTATE, "cavgym_rollout needs an on-device agent for every body");
+  if ((rc = refuse_dense_with_params(eng, "cavgym_rollout"))) return rc;
   if (n_steps == 0) return CAV_OK;
   if (eng->dense) {
     const StepIO<double> io64{nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, 0};
@@ -917,8 +966,16 @@ int cavgym_rollout(CavEngine* eng, int n_steps, int auto_reset, cudaStream_t str
     eng->t_global += n_steps;
     return CAV_OK;
   }
-  if (eng->dtype == CAV_F64) small_launchers<double>(eng->m)->rollout(eng->sc64, eng->buf64, eng->t_global, n_steps, auto_reset, stream);
-  else small_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
+  if (eng->agent_params_set()) {
+    if (eng->dtype == CAV_F64)
+      params_launchers<double>(eng->m)->rollout(eng->sc64, eng->buf64, agent_params<double>(eng), eng->t_global, n_steps, auto_reset, stream);
+    else
+      params_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, agent_params<float>(eng), eng->t_global, n_steps, auto_reset, stream);
+  } else if (eng->dtype == CAV_F64) {
+    small_launchers<double>(eng->m)->rollout(eng->sc64, eng->buf64, eng->t_global, n_steps, auto_reset, stream);
+  } else {
+    small_launchers<float>(eng->m)->rollout(eng->sc32, eng->buf32, eng->t_global, n_steps, auto_reset, stream);
+  }
   rc = launch_check(eng, "rollout kernel");
   if (rc) return rc;
   eng->t_global += n_steps;
@@ -932,6 +989,7 @@ int cavgym_rollout_record(CavEngine* eng, int n_steps, int auto_reset, const Cav
   if (rc) return rc;
   if (n_steps < 0) return fail(CAV_EINVAL, "n_steps must be >= 0");
   if (eng->has_external) return fail(CAV_ESTATE, "cavgym_rollout_record needs an on-device agent for every body");
+  if ((rc = refuse_dense_with_params(eng, "cavgym_rollout_record"))) return rc;
   if (n_steps == 0) return CAV_OK;
   rc = eng->dtype == CAV_F64 ? rollout_record_typed(eng, eng->sc64, eng->buf64, *rec, n_steps, auto_reset, stream)
                              : rollout_record_typed(eng, eng->sc32, eng->buf32, *rec, n_steps, auto_reset, stream);
@@ -953,6 +1011,8 @@ int cavgym_rollout_until(CavEngine* eng, int n_steps, double level, uint64_t sal
   if (eng->has_external) return fail(CAV_ESTATE, "cavgym_rollout_until needs an on-device agent for every body");
   if (eng->dense) return fail(CAV_ESTATE, "cavgym_rollout_until runs on the thread-per-environment path only (at most CAV_SMALL_M bodies, "
                                           "cavgym_set_dense_path off)");
+  if (eng->agent_params_set())
+    return fail(CAV_ESTATE, "cavgym_rollout_until does not read per-env agent parameters: clear them (cavgym_set_agent_params) first");
   if (n_steps == 0) return CAV_OK;
   if (eng->dtype == CAV_F64)
     rollout_until_launcher<double>(eng->m)(eng->sc64, eng->buf64, (double*)score, status, level, salt, eng->t_global, n_steps, stream);
@@ -961,6 +1021,51 @@ int cavgym_rollout_until(CavEngine* eng, int n_steps, double level, uint64_t sal
   rc = launch_check(eng, "rollout until kernel");
   if (rc) return rc;
   eng->t_global += n_steps;
+  return CAV_OK;
+}
+
+int cavgym_set_agent_params(CavEngine* eng, const double* epsilon, const void* threshold, cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!epsilon && !threshold) {
+    eng->epsilon_set = eng->threshold_set = false;
+    return CAV_OK;
+  }
+  if (eng->m > CAV_SMALL_M)
+    return fail(CAV_ESTATE, "per-env agent parameters are read by the thread-per-environment kernels only (at most CAV_SMALL_M bodies)");
+  uint32_t eps_rows = 0, thr_rows = 0;   // bit b: body b's agent reads that row
+  for (int b = 0; b < eng->m; ++b) {
+    const int agent = eng->bodies[(size_t)b].agent;
+    if (agent == CAV_AGENT_RANDOM || agent == CAV_AGENT_RANDOM_CONSTRAINED) eps_rows |= 1u << b;
+    if (agent == CAV_AGENT_PROXIMITY || agent == CAV_AGENT_ELECTION) thr_rows |= 1u << b;
+  }
+  const size_t count = (size_t)eng->m * (size_t)eng->n;
+  if (!eng->d_param_flags) {
+    if ((rc = dev_alloc(eng, &eng->d_param_flags, 1))) return rc;
+    if ((rc = dev_alloc(eng, &eng->d_epsilon, count, false))) return rc;
+    char* thr = nullptr;
+    if ((rc = dev_alloc(eng, &thr, count * eng->real_size(), false))) return rc;
+    eng->d_threshold = thr;
+  }
+  // the caller's arrays are checked before they are copied: a refused call leaves the engine's parameters as they were
+  CUDA_TRY(cudaMemsetAsync(eng->d_param_flags, 0, sizeof(unsigned int), stream));
+  if (eng->dtype == CAV_F64)
+    check_agent_params_kernel<double><<<148 * 4, 256, 0, stream>>>(epsilon, (const double*)threshold, eng->n, eng->m, eps_rows, thr_rows,
+                                                                  eng->d_param_flags);
+  else
+    check_agent_params_kernel<float><<<148 * 4, 256, 0, stream>>>(epsilon, (const float*)threshold, eng->n, eng->m, eps_rows, thr_rows,
+                                                                 eng->d_param_flags);
+  if ((rc = launch_check(eng, "agent parameter check kernel"))) return rc;
+  unsigned int bad = 0;
+  CUDA_TRY(cudaMemcpyAsync(&bad, eng->d_param_flags, sizeof(bad), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaStreamSynchronize(stream));
+  if (bad & 1u) return fail(CAV_EINVAL, "epsilon outside [0, 1] (or NaN) in a row a RandomAgent / RandomConstrainedAgent reads");
+  if (bad & 2u) return fail(CAV_EINVAL, "threshold not finite and > 0 in a row a ProximityAgent / ElectionAgent reads");
+  if (epsilon) CUDA_TRY(cudaMemcpyAsync(eng->d_epsilon, epsilon, count * sizeof(double), cudaMemcpyDeviceToDevice, stream));
+  if (threshold) CUDA_TRY(cudaMemcpyAsync(eng->d_threshold, threshold, count * eng->real_size(), cudaMemcpyDeviceToDevice, stream));
+  CUDA_TRY(cudaStreamSynchronize(stream));
+  eng->epsilon_set = epsilon != nullptr;
+  eng->threshold_set = threshold != nullptr;
   return CAV_OK;
 }
 
@@ -1016,6 +1121,7 @@ int cavgym_step_host(CavEngine* eng, const void* actions, void* state_out, void*
   int rc = check_engine(eng);
   if (rc) return rc;
   if (!actions && eng->has_external) return fail(CAV_EINVAL, "actions is NULL but a body has CAV_AGENT_EXTERNAL");
+  if ((rc = refuse_dense_with_params(eng, "cavgym_step_host"))) return rc;
   const int64_t n = eng->n, m = eng->m;
   const size_t rs = eng->real_size();
   if ((rc = host_setup(eng))) return rc;
@@ -1093,6 +1199,8 @@ int cavgym_step_host_f32(CavEngine* eng, const float* actions, float* state_out,
   if (rc) return rc;
   if (eng->dtype != CAV_F64) return fail(CAV_ESTATE, "the float32 wire format is for fp64 engines; a float32 engine uses cavgym_step_host");
   if (eng->dense) return fail(CAV_ESTATE, "the float32 wire format is implemented by the thread-per-environment kernels (at most CAV_SMALL_M bodies)");
+  if (eng->agent_params_set())
+    return fail(CAV_ESTATE, "the float32 wire format does not read per-env agent parameters: clear them (cavgym_set_agent_params) first");
   if (!actions && eng->has_external) return fail(CAV_EINVAL, "actions is NULL but a body has CAV_AGENT_EXTERNAL");
   if ((rc = host_setup(eng))) return rc;
   if (eng->caller_work_pending) CUDA_TRY(cudaDeviceSynchronize());

@@ -163,6 +163,14 @@ struct CtaPhase {
   __device__ __forceinline__ void operator()() const { if (on) { __syncwarp(); __syncthreads(); } }
 };
 
+// `tester` gives the transition the on-device agents' parameters: body b's RandomAgent / RandomConstrainedAgent epsilon
+// (template.py:52-62, pedestrian.py:72-75) and ProximityAgent / ElectionAgent distance threshold (pedestrian.py:78-91) for
+// env e.  SceneTester reads the scenario's values, the same for every env; EnvTester (kernels_params.cuh) reads per-env ones.
+struct SceneTester {
+  template <typename R> __device__ __forceinline__ double epsilon(const DevBody<R>& body, int, int64_t, int64_t) const { return body.epsilon; }
+  template <typename R> __device__ __forceinline__ R threshold(const DevBody<R>& body, int, int64_t, int64_t) const { return body.threshold; }
+};
+
 // `moved(env)` is called once, right after body.step: a kernel that stages state in shared memory writes the new
 // state there at that point, so x, y, v, theta need not stay in registers through the geometry.
 //
@@ -193,31 +201,34 @@ struct CtaPhase {
 #endif
 
 #define CAV_BODY_LOOP _Pragma("unroll")
-template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase>
+template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
+          typename Tester = SceneTester>
 __device__ __forceinline__ void transition_unrolled(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                                     EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                                    Sink moved = Sink(), Phase phase = Phase()) {
+                                                    Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
 #include "transition_body.inc"
 }
 #undef CAV_BODY_LOOP
 
 #define CAV_BODY_LOOP _Pragma("unroll 1")
-template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase>
+template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
+          typename Tester = SceneTester>
 __device__ __forceinline__ void transition_rolled(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                                   EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                                  Sink moved = Sink(), Phase phase = Phase()) {
+                                                  Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
 #include "transition_body.inc"
 }
 #undef CAV_BODY_LOOP
 
-template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase>
+template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
+          typename Tester = SceneTester>
 __device__ __forceinline__ void transition(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                            EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                           Sink moved = Sink(), Phase phase = Phase()) {
+                                           Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
   if constexpr ((GENERIC && M >= CAV_ROLLED_FROM_M) || (!GENERIC && AGENTS && M >= CAV_ROLLED_HOMOGENEOUS_FROM_M) ||
                 (!GENERIC && !AGENTS && M >= CAV_ROLLED_HOMOGENEOUS_REPLAY_FROM_M) ||
-                (AGENTS && CAV_ROLL_AGENTS != 0 && M >= 2)) transition_rolled<R, M, AGENTS, GENERIC, Sink, Phase>(sc, buf, e, t_global, env, ext, out, moved, phase);
-  else transition_unrolled<R, M, AGENTS, GENERIC, Sink, Phase>(sc, buf, e, t_global, env, ext, out, moved, phase);
+                (AGENTS && CAV_ROLL_AGENTS != 0 && M >= 2)) transition_rolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester>(sc, buf, e, t_global, env, ext, out, moved, phase, tester);
+  else transition_unrolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester>(sc, buf, e, t_global, env, ext, out, moved, phase, tester);
 }
 
 // reporting.analyse_episode (reporting.py:227-243) for an env whose episode just ended.  The lanes of a warp that end their

@@ -130,6 +130,7 @@ class BatchedCAVEnv:
         self.tangent = torch.zeros(n, dtype=torch.uint8, device=self.device)
         self._keep = {}
         self._host_seen = {}
+        self._agent_params = (None, None)
 
     # ---- plumbing ----------------------------------------------------------------------
     def _view(self, getter, shape, typestr):
@@ -238,6 +239,47 @@ class BatchedCAVEnv:
         _native.check(self._lib.cavgym_rollout_until(self._handle, int(n_steps), float(level), int(salt) % (1 << 64), _ptr(score),
                                                      _ptr(status), self._stream()))
         return status
+
+    # ---- per-env tester parameters -------------------------------------------------------------
+    EPSILON_AGENTS = (_abi.CAV_AGENT_RANDOM, _abi.CAV_AGENT_RANDOM_CONSTRAINED)
+    THRESHOLD_AGENTS = (_abi.CAV_AGENT_PROXIMITY, _abi.CAV_AGENT_ELECTION)
+
+    def agent_rows(self):
+        """(epsilon rows, threshold rows): the bodies whose agent reads row b of set_agent_params' epsilon / threshold."""
+        kinds = [int(self.compiled.struct.bodies[b].agent) for b in range(self.num_bodies)]
+        return ([b for b, k in enumerate(kinds) if k in self.EPSILON_AGENTS],
+                [b for b, k in enumerate(kinds) if k in self.THRESHOLD_AGENTS])
+
+    def set_agent_params(self, epsilon=None, threshold=None):
+        """Per-env tester parameters (cavgym_set_agent_params): env e's body b uses epsilon[b, e] instead of its RandomAgent /
+        RandomConstrainedAgent epsilon and threshold[b, e] instead of its ProximityAgent / ElectionAgent distance threshold.
+        Each is [M, N] of anything convertible (epsilon is kept in float64, threshold in the engine's dtype) or None for the
+        scenario's value; both None clears them.  Only the rows of bodies with such an agent are read (agent_rows()); other
+        rows may hold anything, NaN included.  ValueError, before any call, for a wrong shape or a read row outside
+        epsilon in [0, 1] / threshold > 0 and finite.  The values belong to the env slots: reset, auto-reset, load_envs and
+        fork leave them in place.  While they are set, step_host with float32 buffers, rollout_until and the warp-per-env
+        path (set_dense_path) refuse to run."""
+        m, n = self.num_bodies, self.num_envs
+        eps_rows, thr_rows = self.agent_rows()
+        eps = None if epsilon is None else torch.as_tensor(epsilon).to(device=self.device, dtype=torch.float64).contiguous()
+        thr = None if threshold is None else torch.as_tensor(threshold).to(device=self.device, dtype=self.dtype).contiguous()
+        for name, tensor in (("epsilon", eps), ("threshold", thr)):
+            if tensor is not None and tuple(tensor.shape) != (m, n):
+                raise ValueError(f"{name} must have shape {(m, n)}, got {tuple(tensor.shape)}")
+        if eps is not None and eps_rows:
+            read = eps[eps_rows]
+            if not bool(((read >= 0) & (read <= 1)).all()):
+                raise ValueError(f"epsilon must be in [0, 1] in the rows {eps_rows} (bodies with a random agent)")
+        if thr is not None and thr_rows:
+            read = thr[thr_rows]
+            if not bool(((read > 0) & torch.isfinite(read)).all()):
+                raise ValueError(f"threshold must be > 0 and finite in the rows {thr_rows} (bodies with a proximity / election agent)")
+        _native.check(self._lib.cavgym_set_agent_params(self._handle, _ptr(eps), _ptr(thr), self._stream()))
+        self._agent_params = (None if eps is None else eps.clone(), None if thr is None else thr.clone())
+
+    def agent_params(self):
+        """(epsilon, threshold) as last set by set_agent_params: [M, N] device tensors, or None where unset."""
+        return self._agent_params
 
     def replay(self, actions, record=("state", "reward", "done", "winner", "tangent")):
         """Replay joint actions [T,M,2,N] in one launch; returns the recorded trajectories as a dict."""
@@ -416,17 +458,23 @@ class BatchedCAVEnv:
     def state_dict(self):
         """Checkpoint of the whole engine: every env (as CPU bytes), t_global, the raw counters, seed, shard, tau and the
         scenario fingerprint.  Tensors, ints, floats and strings only (torch.load with weights_only reads it).  The
-        episode-log ring is not included: drain it first."""
+        episode-log ring is not included: drain it first.  Per-env tester parameters (set_agent_params) are included as
+        "agent_epsilon" / "agent_threshold" CPU tensors [M, N] where they are set, and absent otherwise."""
         state = self._engine_state()
         envs = self.save_envs().cpu()
-        return {"version": int(state.version), "dtype": str(self.dtype).replace("torch.", ""), "num_envs": int(state.n),
-                "num_bodies": int(state.m), "seed": int(state.seed), "env_offset": int(state.shard), "tau": float(state.tau),
-                "t_global": int(state.t_global), "counters": torch.tensor(list(state.counters), dtype=torch.int64),
-                "fingerprint": f"{state.fingerprint:016x}", "envs": envs.data}
+        out = {"version": int(state.version), "dtype": str(self.dtype).replace("torch.", ""), "num_envs": int(state.n),
+               "num_bodies": int(state.m), "seed": int(state.seed), "env_offset": int(state.shard), "tau": float(state.tau),
+               "t_global": int(state.t_global), "counters": torch.tensor(list(state.counters), dtype=torch.int64),
+               "fingerprint": f"{state.fingerprint:016x}", "envs": envs.data}
+        for key, value in zip(("agent_epsilon", "agent_threshold"), self._agent_params):
+            if value is not None:
+                out[key] = value.cpu()
+        return out
 
     def load_state_dict(self, state_dict):
         """Continue a checkpoint of state_dict(): this engine must have the same scenario, dtype, env count, seed and
-        env_offset (ValueError otherwise); tau is taken from the checkpoint."""
+        env_offset (ValueError otherwise); tau is taken from the checkpoint.  The per-env tester parameters are set from
+        the checkpoint's "agent_epsilon" / "agent_threshold", or cleared where it has none, so that it continues bit for bit."""
         sd, mine = state_dict, self._engine_state()
         want = {"version": int(mine.version), "fingerprint": f"{mine.fingerprint:016x}",
                 "dtype": str(self.dtype).replace("torch.", ""), "num_envs": int(mine.n), "num_bodies": int(mine.m),
@@ -443,6 +491,8 @@ class BatchedCAVEnv:
         snapshot = EnvSnapshot(torch.as_tensor(sd["envs"]), self._layout(self.num_envs))
         if tuple(snapshot.data.shape) != (int(snapshot.layout.total_bytes),) or snapshot.data.dtype != torch.uint8:
             raise ValueError("checkpoint envs do not have the size this engine's layout gives")
+        epsilon, threshold = sd.get("agent_epsilon"), sd.get("agent_threshold")
+        self.set_agent_params(epsilon, threshold)   # validated before the engine state is touched
         _native.check(self._lib.cavgym_load_engine(self._handle, C.byref(state)))
         self.load_envs(snapshot)
 

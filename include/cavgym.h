@@ -21,7 +21,8 @@
  * Errors: every call returns 0 or a negative CAV_E* code and never throws;
  * cavgym_last_error() gives the message of the calling thread's last failure.
  * One engine per device; an engine is not thread-safe.  No call synchronises the
- * host with the device except cavgym_stats, cavgym_error_count and the *_host calls.
+ * host with the device except cavgym_stats, cavgym_error_count, cavgym_set_agent_params
+ * and the *_host calls.
  */
 #ifndef CAVGYM_H
 #define CAVGYM_H
@@ -262,9 +263,28 @@ int cavgym_rollout_record(CavEngine* engine, int n_steps, int auto_reset, const 
  * just discarded.  An ordinary launch on `stream`.  n_steps = 0 does nothing.
  * CAV_EINVAL: NULL engine, score or status, n_steps < 0, NaN level, a scenario no tester can win (terminate_ego_zones off
  * or no Pedestrian body).  CAV_ESTATE: a body with CAV_AGENT_EXTERNAL, or the warp-per-environment path (more than
- * CAV_SMALL_M bodies, or cavgym_set_dense_path(1)). */
+ * CAV_SMALL_M bodies, or cavgym_set_dense_path(1)), or per-env agent parameters set (cavgym_set_agent_params). */
 int cavgym_rollout_until(CavEngine* engine, int n_steps, double level, uint64_t salt, void* score, uint8_t* status,
                          cudaStream_t stream);
+
+/* Per-env tester parameters, so that one batch can sweep them: env e's body b uses epsilon[b][e] where the scenario's
+ * RandomAgent / RandomConstrainedAgent epsilon (CavBody.agent_epsilon; template.py:52-62, pedestrian.py:72-75) would be used,
+ * and threshold[b][e] where its ProximityAgent / ElectionAgent distance_threshold (CavBody.agent_threshold;
+ * pedestrian.py:78-91) would be.
+ *   epsilon    device double[M][N] (double in both engine types, as agent_epsilon), nullable
+ *   threshold  device real[M][N], nullable
+ * A NULL array means the scenario's value; both NULL clears the parameters and returns the engine to its plain kernels.
+ * Row b of epsilon is read only where body b's agent is CAV_AGENT_RANDOM or CAV_AGENT_RANDOM_CONSTRAINED, row b of threshold
+ * only where it is CAV_AGENT_PROXIMITY or CAV_AGENT_ELECTION; other rows may hold anything (NaN included).  The rows that are
+ * read must hold epsilon in [0, 1] and threshold > 0 and finite (config.py's ranges): CAV_EINVAL otherwise, and the engine's
+ * parameters are left as they were.  The arrays are copied into engine-owned buffers; agent kinds stay the scenario's.
+ * The parameters belong to the env SLOTS: cavgym_reset, auto-reset, cavgym_load_envs and cavgym_fork_envs do not move them,
+ * and cavgym_save_engine does not carry them.  Philox streams are unchanged: only the decisions draw < epsilon and
+ * distance < threshold differ.  Honoured by cavgym_step and cavgym_step_host with on-device agents, cavgym_rollout and
+ * cavgym_rollout_record.  While parameters are set, cavgym_step_host_f32 and cavgym_rollout_until return CAV_ESTATE, and
+ * so does any stepping call on the warp-per-environment path (cavgym_set_dense_path(1)).
+ * CAV_ESTATE also for parameters on a scenario of more than CAV_SMALL_M bodies.  Synchronises `stream`. */
+int cavgym_set_agent_params(CavEngine* engine, const double* epsilon, const void* threshold, cudaStream_t stream);
 
 /* Replayed joint actions, n_steps transitions in one launch:
  * actions real[T][M][2][N]; trajectory outputs (each nullable) state real[T][M][4][N],
