@@ -97,6 +97,7 @@ PROTOTYPES = {
     "cavgym_rollout_record": (C.c_int, [c_engine_p, C.c_int, C.c_int, C.POINTER(CavRolloutRecord), c_stream]),
     "cavgym_rollout_until": (C.c_int, [c_engine_p, C.c_int, C.c_double, C.c_uint64, C.c_void_p, C.c_void_p, c_stream]),
     "cavgym_set_agent_params": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, c_stream]),
+    "cavgym_regenerate_episodes": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_int, C.POINTER(CavRolloutRecord), c_stream]),
     "cavgym_replay": (C.c_int, [c_engine_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, c_stream]),
     "cavgym_step_host": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "cavgym_step_host_f32": (C.c_int, [c_engine_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -2,7 +2,7 @@
 
     python -m cavgym_b200.csrc.build [--force] [--jobs N]
 
-One translation unit per body count (small_mK.cu, record_mK.cu, until_mK.cu, params_mK.cu) so the kernels compile in parallel.
+One translation unit per body count (small_mK.cu, record_mK.cu, until_mK.cu, params_mK.cu, regen_mK.cu) so the kernels compile in parallel.
 -fmad=false keeps the fp64 arithmetic in the reference's operation order (no FMA contraction).
 """
 import argparse
@@ -35,7 +35,7 @@ EXTRA = os.environ.get("CAVGYM_NVCC_FLAGS", "").split()
 
 
 def compile_one(src, force, verbose):
-    stub = bool(ONLY_M) and src.startswith(("small_m", "record_m", "until_m", "params_m")) and int(src.split("_m")[1][:-3]) not in ONLY_M
+    stub = bool(ONLY_M) and src.startswith(("small_m", "record_m", "until_m", "params_m", "regen_m")) and int(src.split("_m")[1][:-3]) not in ONLY_M
     obj = os.path.join(OBJ_DIR, src[:-3] + (".stub.o" if stub else ".o"))
     src_path = os.path.join(HERE, src)
     if not force and not EXTRA and os.path.isfile(obj) and os.path.getmtime(obj) >= max(os.path.getmtime(src_path), headers_mtime()):

@@ -23,6 +23,7 @@
 #include "kernels_snapshot.cuh"
 #include "kernels_until.cuh"
 #include "kernels_params.cuh"
+#include "kernels_regen.cuh"
 
 namespace cav {
 
@@ -35,7 +36,9 @@ namespace cav {
   extern const RolloutUntilLauncher<double> kUntilF64M##K; \
   extern const RolloutUntilLauncher<float> kUntilF32M##K; \
   extern const ParamsLaunchers<double> kParamsF64M##K; \
-  extern const ParamsLaunchers<float> kParamsF32M##K;
+  extern const ParamsLaunchers<float> kParamsF32M##K; \
+  extern const RegenerateLauncher<double> kRegenF64M##K; \
+  extern const RegenerateLauncher<float> kRegenF32M##K;
 CAV_FOR_EACH_M(CAV_DECLARE)
 #undef CAV_DECLARE
 
@@ -105,6 +108,34 @@ template <> const ParamsLaunchers<float>* params_launchers<float>(int m) {
 #undef CAV_CASE
     default: return nullptr;
   }
+}
+
+template <> RegenerateLauncher<double> regenerate_launcher<double>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kRegenF64M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+template <> RegenerateLauncher<float> regenerate_launcher<float>(int m) {
+  switch (m) {
+#define CAV_CASE(K) case K: return kRegenF32M##K;
+    CAV_FOR_EACH_M(CAV_CASE)
+#undef CAV_CASE
+    default: return nullptr;
+  }
+}
+
+// cavgym_regenerate_episodes' range check of the caller's keys: bit 0 of *bad for a global env id outside [0, 2^40) (the ids
+// cavgym_set_shard admits), bit 1 for a negative episode number.
+__global__ void check_regen_keys_kernel(const int64_t* env_ids, const int32_t* episodes, int64_t n, unsigned int* bad) {
+  unsigned int flags = 0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    if (env_ids[i] < 0 || env_ids[i] >= ((int64_t)1 << 40)) flags |= 1u;
+    if (episodes[i] < 0) flags |= 2u;
+  }
+  if (flags) atomicOr(bad, flags);
 }
 
 static thread_local std::string g_error;
@@ -516,6 +547,7 @@ struct CavEngine {
   void* d_threshold = nullptr;
   unsigned int* d_param_flags = nullptr;
   bool epsilon_set = false, threshold_set = false;
+  unsigned int* d_regen_flags = nullptr;   // cavgym_regenerate_episodes' key check, allocated on first use
 
   bool agent_params_set() const { return epsilon_set || threshold_set; }
   size_t real_size() const { return dtype == CAV_F64 ? 8 : 4; }
@@ -1020,6 +1052,49 @@ int cavgym_rollout_until(CavEngine* eng, int n_steps, double level, uint64_t sal
     rollout_until_launcher<float>(eng->m)(eng->sc32, eng->buf32, (float*)score, status, level, salt, eng->t_global, n_steps, stream);
   rc = launch_check(eng, "rollout until kernel");
   if (rc) return rc;
+  eng->t_global += n_steps;
+  return CAV_OK;
+}
+
+int cavgym_regenerate_episodes(CavEngine* eng, const int64_t* env_ids, const int32_t* episodes, int n_steps, const CavRolloutRecord* rec,
+                               cudaStream_t stream) {
+  int rc = check_engine(eng);
+  if (rc) return rc;
+  if (!env_ids || !episodes) return fail(CAV_EINVAL, "env_ids/episodes is NULL");
+  if (n_steps < 0) return fail(CAV_EINVAL, "n_steps must be >= 0");
+  if (eng->has_external)
+    return fail(CAV_ESTATE, "cavgym_regenerate_episodes needs an on-device agent for every body (external actions came from the caller)");
+  for (int b = 0; b < eng->m; ++b)
+    if (eng->bodies[(size_t)b].agent == CAV_AGENT_ELECTION)
+      return fail(CAV_ESTATE, "cavgym_regenerate_episodes: an election outlives episodes, so an episode depends on the ones before it");
+  if (eng->dense)
+    return fail(CAV_ESTATE, "cavgym_regenerate_episodes runs on the thread-per-environment path only (at most CAV_SMALL_M bodies, "
+                            "cavgym_set_dense_path off)");
+  if (eng->buf64.uni_override || eng->buf64.spawn_override)
+    return fail(CAV_ESTATE, "cavgym_regenerate_episodes draws from the engine's random streams: clear the uniform / spawn overrides");
+  if (!eng->d_regen_flags && (rc = dev_alloc(eng, &eng->d_regen_flags, 1))) return rc;
+  CUDA_TRY(cudaMemsetAsync(eng->d_regen_flags, 0, sizeof(unsigned int), stream));
+  check_regen_keys_kernel<<<148 * 4, 256, 0, stream>>>(env_ids, episodes, eng->n, eng->d_regen_flags);
+  if ((rc = launch_check(eng, "regeneration key check kernel"))) return rc;
+  unsigned int bad = 0;
+  CUDA_TRY(cudaMemcpyAsync(&bad, eng->d_regen_flags, sizeof(bad), cudaMemcpyDeviceToHost, stream));
+  CUDA_TRY(cudaStreamSynchronize(stream));
+  if (bad & 1u) return fail(CAV_EINVAL, "env id outside [0, 2^40)");
+  if (bad & 2u) return fail(CAV_EINVAL, "negative episode number");
+  const CavRolloutRecord none{};
+  const CavRolloutRecord& r = rec ? *rec : none;
+  if (eng->dtype == CAV_F64) {
+    const RolloutRecord<double> slabs{(double*)r.observation, (double*)r.action, (double*)r.state, (double*)r.reward, r.done, r.winner,
+                                      r.tangent, r.timestep};
+    regenerate_launcher<double>(eng->m)(eng->sc64, eng->buf64, slabs, agent_params<double>(eng), env_ids, episodes, eng->t_global,
+                                        n_steps, stream);
+  } else {
+    const RolloutRecord<float> slabs{(float*)r.observation, (float*)r.action, (float*)r.state, (float*)r.reward, r.done, r.winner,
+                                     r.tangent, r.timestep};
+    regenerate_launcher<float>(eng->m)(eng->sc32, eng->buf32, slabs, agent_params<float>(eng), env_ids, episodes, eng->t_global,
+                                       n_steps, stream);
+  }
+  if ((rc = launch_check(eng, "regeneration kernel"))) return rc;
   eng->t_global += n_steps;
   return CAV_OK;
 }

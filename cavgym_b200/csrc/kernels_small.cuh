@@ -139,10 +139,11 @@ __device__ __forceinline__ void write_outputs(const EnvBuffers<R>& buf, const St
 // actions, outputs, latching and scoring.  Returns true if the episode ended in this step.  One output site: frozen
 // (finished, not yet reset) envs report reward 0 and their latched done / winner through the same stores.
 // `ghost`: the lane steps a COPY of env e to keep its warp whole (rollout_kernel); nothing it does may be seen.
-template <typename R, int M, bool AGENTS, bool GENERIC, typename Phase = NoPhase, typename Tester = SceneTester>
+template <typename R, int M, bool AGENTS, bool GENERIC, typename Phase = NoPhase, typename Tester = SceneTester, typename Key = ShardKey>
 __device__ __forceinline__ bool advance(const DevScenario<R>& sc, const EnvBuffers<R>& buf, const StepIO<R>& io, int64_t e,
                                         int64_t t_global, EnvRegs<R, M>& env, const R (&ext)[M][2], Phase phase = Phase(),
-                                        const bool ghost = false, R* reward_sink = nullptr, const Tester tester = Tester()) {
+                                        const bool ghost = false, R* reward_sink = nullptr, const Tester tester = Tester(),
+                                        const Key key = Key()) {
   StepResult<R, M> res;
   bool ended = false;
   if (CAV_UNLIKELY(env.done != 0)) {  // frozen until reset
@@ -152,11 +153,11 @@ __device__ __forceinline__ bool advance(const DevScenario<R>& sc, const EnvBuffe
     res.winner = env.winner;
     res.tangent = false;
   } else {
-    transition<R, M, AGENTS, GENERIC, NoSink, Phase, Tester>(sc, buf, e, t_global, env, ext, res, NoSink(), phase, tester);
+    transition<R, M, AGENTS, GENERIC, NoSink, Phase, Tester, Key>(sc, buf, e, t_global, env, ext, res, NoSink(), phase, tester, key);
     if (!ghost) {
       if (CAV_UNLIKELY(res.invalid)) buf.err[e] = 1;
       if (CAV_UNLIKELY(res.tangent)) count_tangent(buf.stats);
-      if (CAV_UNLIKELY(env.done != 0)) score_episode<R, M>(buf, env, e, AGENTS ? env.episode : -1);
+      if (CAV_UNLIKELY(env.done != 0)) score_episode<R, M, Key>(buf, env, e, AGENTS ? env.episode : -1, key);
     }
     ended = env.done != 0;
   }

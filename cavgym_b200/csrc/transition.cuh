@@ -171,6 +171,13 @@ struct SceneTester {
   template <typename R> __device__ __forceinline__ R threshold(const DevBody<R>& body, int, int64_t, int64_t) const { return body.threshold; }
 };
 
+// `key` gives the global env id that keys env e's Philox draws (spawns in reset_env, agents in the transition) and that its
+// episode rows carry.  ShardKey is slot e of the engine's shard; SlotKey (kernels_regen.cuh) is an id the caller gave for the
+// slot, so that a slot replays the episodes of another env.
+struct ShardKey {
+  template <typename R> __device__ __forceinline__ int64_t operator()(const EnvBuffers<R>& buf, int64_t e) const { return buf.shard + e; }
+};
+
 // `moved(env)` is called once, right after body.step: a kernel that stages state in shared memory writes the new
 // state there at that point, so x, y, v, theta need not stay in registers through the geometry.
 //
@@ -202,33 +209,35 @@ struct SceneTester {
 
 #define CAV_BODY_LOOP _Pragma("unroll")
 template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
-          typename Tester = SceneTester>
+          typename Tester = SceneTester, typename Key = ShardKey>
 __device__ __forceinline__ void transition_unrolled(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                                     EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                                    Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
+                                                    Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester(),
+                                                    Key key = Key()) {
 #include "transition_body.inc"
 }
 #undef CAV_BODY_LOOP
 
 #define CAV_BODY_LOOP _Pragma("unroll 1")
 template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
-          typename Tester = SceneTester>
+          typename Tester = SceneTester, typename Key = ShardKey>
 __device__ __forceinline__ void transition_rolled(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                                   EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                                  Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
+                                                  Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester(),
+                                                  Key key = Key()) {
 #include "transition_body.inc"
 }
 #undef CAV_BODY_LOOP
 
 template <typename R, int M, bool AGENTS, bool GENERIC, typename Sink = NoSink, typename Phase = NoPhase,
-          typename Tester = SceneTester>
+          typename Tester = SceneTester, typename Key = ShardKey>
 __device__ __forceinline__ void transition(const DevScenario<R>& sc, const EnvBuffers<R>& buf, int64_t e, int64_t t_global,
                                            EnvRegs<R, M>& env, const R (&ext)[M][2], StepResult<R, M>& out,
-                                           Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester()) {
+                                           Sink moved = Sink(), Phase phase = Phase(), Tester tester = Tester(), Key key = Key()) {
   if constexpr ((GENERIC && M >= CAV_ROLLED_FROM_M) || (!GENERIC && AGENTS && M >= CAV_ROLLED_HOMOGENEOUS_FROM_M) ||
                 (!GENERIC && !AGENTS && M >= CAV_ROLLED_HOMOGENEOUS_REPLAY_FROM_M) ||
-                (AGENTS && CAV_ROLL_AGENTS != 0 && M >= 2)) transition_rolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester>(sc, buf, e, t_global, env, ext, out, moved, phase, tester);
-  else transition_unrolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester>(sc, buf, e, t_global, env, ext, out, moved, phase, tester);
+                (AGENTS && CAV_ROLL_AGENTS != 0 && M >= 2)) transition_rolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester, Key>(sc, buf, e, t_global, env, ext, out, moved, phase, tester, key);
+  else transition_unrolled<R, M, AGENTS, GENERIC, Sink, Phase, Tester, Key>(sc, buf, e, t_global, env, ext, out, moved, phase, tester, key);
 }
 
 // reporting.analyse_episode (reporting.py:227-243) for an env whose episode just ended.  The lanes of a warp that end their
@@ -281,21 +290,22 @@ __device__ __noinline__ void score_episode(unsigned long long* stats, int32_t t_
 }
 
 // `episode` = the env's episode number if the kernel carries it in registers (on-device agents), else -1: read it back.
-template <typename R, int M>
-__device__ __forceinline__ void score_episode(const EnvBuffers<R>& buf, const EnvRegs<R, M>& env, int64_t e, int32_t episode = -1) {
+template <typename R, int M, typename Key = ShardKey>
+__device__ __forceinline__ void score_episode(const EnvBuffers<R>& buf, const EnvRegs<R, M>& env, int64_t e, int32_t episode = -1,
+                                              Key key = Key()) {
   long long sum = 0;
 #pragma unroll
   for (int b = 1; b < M; ++b) sum += env.live[b];
-  EpisodeLog log{buf.ep_log, buf.ep_log_count, buf.ep_log_capacity, buf.shard + e, episode};
+  EpisodeLog log{buf.ep_log, buf.ep_log_count, buf.ep_log_capacity, key(buf, e), episode};
   if (buf.ep_log && episode < 0) log.episode = buf.episode[e];
   score_episode<R, M>(buf.stats, env.t_ep, env.winner, sum, log);
 }
 
 // CAVEnv.reset for one env (environment.py:225-229): bodies back to init_state (SpawnPedestrians re-drawn),
 // liveness zeroed, agents reset, on-device noop action.  `init` (nullable) replays given initial states.
-template <typename R, int M>
+template <typename R, int M, typename Key = ShardKey>
 __device__ __forceinline__ void reset_env(const DevScenario<R>& sc, const EnvBuffers<R>& buf, const R* init, int64_t e,
-                                          EnvRegs<R, M>& env) {
+                                          EnvRegs<R, M>& env, Key key = Key()) {
   env.episode += 1;
 #pragma unroll
   for (int b = 0; b < M; ++b) {
@@ -313,7 +323,7 @@ __device__ __forceinline__ void reset_env(const DevScenario<R>& sc, const EnvBuf
         for (int c = 0; c < 5; ++c) u[c] = buf.spawn_override[((int64_t)b * 5 + c) * buf.n + e];
       } else {
         double w[2];
-        const uint64_t g = (uint64_t)(buf.shard + e);
+        const uint64_t g = (uint64_t)key(buf, e);
         draw_block(buf.seed, g, b, KIND_SPAWN0, (uint32_t)env.episode, 0u, w); u[0] = w[0]; u[1] = w[1];
         draw_block(buf.seed, g, b, KIND_SPAWN1, (uint32_t)env.episode, 0u, w); u[2] = w[0]; u[3] = w[1];
         draw_block(buf.seed, g, b, KIND_SPAWN2, (uint32_t)env.episode, 0u, w); u[4] = w[0];

@@ -114,6 +114,7 @@ class BatchedCAVEnv:
                                               int(seed), C.byref(self._handle)))
         if env_offset:
             _native.check(self._lib.cavgym_set_shard(self._handle, int(env_offset)))
+        self.env_offset = int(env_offset)   # global id of env 0
         n, m = self.num_envs, self.num_bodies
         real = "<f8" if self.code == _abi.CAV_F64 else "<f4"
         self.state = self._view(self._lib.cavgym_state_ptr, (m, 4, n), real)
@@ -200,18 +201,136 @@ class BatchedCAVEnv:
         if record is None:
             _native.check(self._lib.cavgym_rollout(self._handle, n_steps, int(bool(auto_reset)), self._stream()))
             return None
+        out, rec = self._record_slabs(n_steps, record)
+        _native.check(self._lib.cavgym_rollout_record(self._handle, n_steps, int(bool(auto_reset)), C.byref(rec), self._stream()))
+        return out
+
+    def _record_names(self, record):
         names = (record,) if isinstance(record, str) else tuple(record)
         unknown = [name for name in names if name not in self.RECORD_FIELDS]
         if unknown:
             raise ValueError(f"unknown record field(s) {unknown}; choose from {tuple(self.RECORD_FIELDS)}")
+        return names
+
+    def _record_slabs(self, n_steps, record):
+        """New device slabs [T, ...] for the RECORD_FIELDS named in `record` (checked), and the CavRolloutRecord of them."""
+        names = self._record_names(record)
         if n_steps < 0:
             raise ValueError("n_steps must be >= 0")
         m, n = self.num_bodies, self.num_envs
         out = {name: torch.empty((n_steps,) + shape(m, n), dtype=dtype or self.dtype, device=self.device)
                for name, (shape, dtype) in self.RECORD_FIELDS.items() if name in names}
-        rec = _abi.CavRolloutRecord(**{name: tensor.data_ptr() for name, tensor in out.items() if tensor.numel()})
-        _native.check(self._lib.cavgym_rollout_record(self._handle, n_steps, int(bool(auto_reset)), C.byref(rec), self._stream()))
+        return out, _abi.CavRolloutRecord(**{name: tensor.data_ptr() for name, tensor in out.items() if tensor.numel()})
+
+    def regenerate_episodes(self, env_ids, episodes, n_steps=None, record=None):
+        """cavgym_regenerate_episodes on this engine: slot e becomes episode episodes[e] of global env env_ids[e] (the `env`
+        and `episode` of an episode row) and steps n_steps times (default max_timesteps) without auto-reset, drawing from the
+        streams of that env and episode, with this engine's per-env tester parameters where set.  The time-out term is
+        decided by this engine's t_global (set_global_timestep) at the first step.  `env_ids` / `episodes` hold N values
+        each.  Returns what rollout(record=...) returns: None, or a dict of new device slabs [T, ...] whose row 0 is the
+        episode's first step.  ValueError, before any call, for a wrong length or an id outside [0, 2^40) or a negative
+        episode.  regenerate() is the form that takes drained rows and returns episodes."""
+        n = self.num_envs
+        ids = torch.as_tensor(np.asarray(env_ids, dtype=np.int64).reshape(-1)).to(self.device).contiguous()
+        eps = torch.as_tensor(np.asarray(episodes, dtype=np.int64).reshape(-1)).to(self.device)
+        if ids.numel() != n or eps.numel() != n:
+            raise ValueError(f"env_ids and episodes must hold {n} values each, got {ids.numel()} and {eps.numel()}")
+        if bool(((ids < 0) | (ids >= (1 << 40))).any()) or bool(((eps < 0) | (eps > np.iinfo(np.int32).max)).any()):
+            raise ValueError("env ids must be in [0, 2^40) and episode numbers in [0, 2^31)")
+        eps = eps.to(torch.int32).contiguous()
+        n_steps = self.max_timesteps if n_steps is None else int(n_steps)
+        if n_steps < 0:
+            raise ValueError("n_steps must be >= 0")
+        out, rec = (None, None) if record is None else self._record_slabs(n_steps, record)
+        _native.check(self._lib.cavgym_regenerate_episodes(self._handle, _ptr(ids), _ptr(eps), n_steps,
+                                                           None if rec is None else C.byref(rec), self._stream()))
         return out
+
+    # share of the free device memory one regenerate() chunk may record into
+    REGENERATE_MEMORY_SHARE = 0.25
+
+    def regenerate(self, rows, record=tuple(RECORD_FIELDS), t_global_start=None, n_steps=None):
+        """The episodes of `rows` — drained episode rows, or any structured array with `env` and `episode` fields — played
+        again on a sibling engine (same compiled scenario, dtype, seed, tau and device, one slot per row) through
+        regenerate_episodes, with this engine's per-env tester parameters of each row's slot (env - env_offset) where they are
+        set.  This engine is not touched.
+
+        t_global_start: the batch-wide step at each episode's first step (an int, or one per row); only the time-out term
+        of the rewards depends on it.  The default, max_timesteps, means "no time-out term", right for every episode that
+        started at or after this engine's step max_timesteps.  n_steps (default max_timesteps) bounds each episode.
+
+        Returns one dict per row, in the order of `rows`, in trajectories.complete_episodes' layout for the recorded
+        fields: "init_state" [M,4] (from "observation"), "actions" [L,M,2] (from "action"), "state" [L,M,4], "reward" [L,M],
+        "done", "winner", "tangent" [L], and "env", "episode", "t_global_start", and "reproduced": whether the regenerated
+        (timesteps, winner, liveness_sum) equal the row's (None if `rows` lacks those fields).  An episode not played from a
+        reset on the engine's own streams (continued after fork or load_envs, or a salted rollout_until stage) comes back
+        with reproduced False; one that has not ended after n_steps has L = n_steps and reproduced False.  Rows are run in
+        chunks whose record fits REGENERATE_MEMORY_SHARE of the free device memory."""
+        rows = np.asarray(rows)
+        if rows.dtype.names is None or "env" not in rows.dtype.names or "episode" not in rows.dtype.names:
+            raise ValueError("rows must be a structured array with 'env' and 'episode' fields (drain_episodes())")
+        rows = rows.reshape(-1)
+        k = rows.size
+        env_ids, episodes = rows["env"].astype(np.int64), rows["episode"].astype(np.int64)
+        if k and (env_ids.min() < 0 or env_ids.max() >= (1 << 40) or episodes.min() < 0 or episodes.max() > np.iinfo(np.int32).max):
+            raise ValueError("rows must have env in [0, 2^40) and episode in [0, 2^31)")
+        starts = np.broadcast_to(np.asarray(self.max_timesteps if t_global_start is None else t_global_start, dtype=np.int64), (k,))
+        if k and starts.min() < 0:
+            raise ValueError("t_global_start must be >= 0")
+        n_steps = self.max_timesteps if n_steps is None else int(n_steps)
+        if n_steps < 0:
+            raise ValueError("n_steps must be >= 0")
+        names = self._record_names(record)
+        state = self._engine_state()
+        slots = env_ids - int(state.shard)
+        params = self._agent_params
+        if any(p is not None for p in params) and k and (slots.min() < 0 or slots.max() >= self.num_envs):
+            raise ValueError(f"per-env tester parameters are set, so every row's env must be one of this engine's "
+                             f"[{int(state.shard)}, {int(state.shard) + self.num_envs})")
+        check = {"timesteps", "winner", "liveness_sum"} <= set(rows.dtype.names)
+        per_step = sum(int(np.prod(shape(self.num_bodies, 1))) * (dtype or self.dtype).itemsize
+                       for name, (shape, dtype) in self.RECORD_FIELDS.items() if name in names)
+        free = torch.cuda.mem_get_info(self.device)[0]
+        chunk = max(1, int(free * self.REGENERATE_MEMORY_SHARE) // max(1, per_step * n_steps))
+        episodes_out = [None] * k
+        for start in np.unique(starts):
+            group = np.flatnonzero(starts == start)
+            for lo in range(0, group.size, chunk):
+                self._regenerate_chunk(rows, group[lo:lo + chunk], int(start), n_steps, names, state, slots, params, check, episodes_out)
+        return episodes_out
+
+    def _regenerate_chunk(self, rows, part, start, n_steps, names, state, slots, params, check, episodes_out):
+        sib = BatchedCAVEnv(None, None, None, num_envs=part.size, dtype=self.dtype, compiled=self.compiled, device=self.device,
+                            seed=int(state.seed))
+        try:
+            sib.set_tangent_tolerance(float(state.tau))
+            if any(p is not None for p in params):
+                index = torch.as_tensor(slots[part], device=self.device)
+                sib.set_agent_params(*(None if p is None else p[:, index] for p in params))
+            sib.set_episode_log(part.size)
+            sib.set_global_timestep(start)
+            rec = sib.regenerate_episodes(rows["env"][part], rows["episode"][part], n_steps, names)
+            got, _ = sib.drain_episodes()
+        finally:
+            sib.close()
+        rec = {name: tensor.cpu().numpy() for name, tensor in rec.items()}
+        found = {(int(r["env"]), int(r["episode"])): r for r in got}
+        for slot, i in enumerate(part):
+            row = rows[i]
+            key = (int(row["env"]), int(row["episode"]))
+            mine = found.get(key)
+            length = n_steps if mine is None else int(mine["timesteps"])
+            episode = {"env": key[0], "episode": key[1], "t_global_start": start}
+            if "observation" in rec:
+                episode["init_state"] = rec["observation"][0, :, :, slot].copy()
+            if "action" in rec:
+                episode["actions"] = np.ascontiguousarray(rec["action"][:length, :, :, slot])
+            for name in ("state", "reward", "done", "winner", "tangent"):
+                if name in rec:
+                    episode[name] = np.ascontiguousarray(rec[name][:length, ..., slot])
+            episode["reproduced"] = None if not check else (
+                mine is not None and all(int(mine[f]) == int(row[f]) for f in ("timesteps", "winner", "liveness_sum")))
+            episodes_out[i] = episode
 
     @property
     def max_timesteps(self):

@@ -6,9 +6,13 @@
                       scoring and auto-reset inside the rollout kernel (cavgym_rollout); the run summary comes from the
                       device counters (cavgym_stats), optionally summed over ranks with one all-reduce; with an
                       `episode_log` the per-episode rows come from the device ring (cavgym_drain_episodes), one per
-                      finished episode, in the reference's episode.log format.
+                      finished episode, in the reference's episode.log format.  With `save_interesting` = K the first K
+                      interesting episodes are regenerated after the run (BatchedCAVEnv.regenerate) and kept in
+                      `interesting`.
 """
 import timeit
+
+import numpy as np
 
 from . import reporting
 from .config import AgentType, Mode
@@ -80,6 +84,8 @@ class BatchedSimulation:
         self.episode_rows = []      # EpisodeResults of every drained episode when an episode log is kept (keep_rows / episode_log)
         self.keep_rows = False
         self.dropped_rows = 0
+        self.save_interesting = 0   # K: regenerate the first K interesting episodes after run() into `interesting`
+        self.interesting = []
 
     def _drain(self, resolution):
         """Per-episode rows from the device ring -> reporting.EpisodeResults, numbered in finishing order (the reference
@@ -87,6 +93,10 @@ class BatchedSimulation:
         (reporting.py:157-158) with NaN for the per-episode wall-clock, which concurrent environments do not have."""
         rows, dropped = self.env.drain_episodes()
         self.dropped_rows += dropped
+        if self.save_interesting:
+            self._note_interesting(rows, dropped)
+        if not (self.keep_rows or self.episode_file):
+            return
         nan = float("nan")
         for row in rows:
             index = self._episodes_logged = getattr(self, "_episodes_logged", 0) + 1
@@ -98,6 +108,33 @@ class BatchedSimulation:
                 self.episode_rows.append((int(row["env"]), int(row["episode"]), result))
             if self.episode_file:
                 self.episode_file.info(result.file_message())
+
+    def _note_interesting(self, rows, dropped):
+        """Keep the first save_interesting rows of tester wins with the t_global of their first step.  With auto-reset an env's
+        next episode starts at the step after its last one ends, so episode j of an env starts at the sum of the lengths of its
+        episodes before j since the run's reset (at t_global 0): every row of the env is needed, so none may be dropped."""
+        if dropped:
+            raise RuntimeError("episode rows were dropped from the device ring: the start steps of later episodes are unknown")
+        env = self.env
+        if not hasattr(self, "_next_start"):
+            self._next_start = np.zeros(env.num_envs, dtype=np.int64)
+        order = np.lexsort((rows["episode"], rows["env"]))
+        slot = rows["env"][order].astype(np.int64) - env.env_offset
+        length = rows["timesteps"][order].astype(np.int64)
+        before = np.cumsum(length) - length                   # within this drain, per env in episode order
+        first = np.r_[True, slot[1:] != slot[:-1]]
+        start = self._next_start[slot] + before - np.maximum.accumulate(np.where(first, before, 0))
+        np.add.at(self._next_start, slot, length)
+        wins = order[rows["winner"][order] > 0]
+        starts = start[rows["winner"][order] > 0]
+        keep = np.argsort(wins, kind="stable")[:max(0, self.save_interesting - sum(len(r) for r, _ in self._hits))]
+        self._hits.append((rows[wins[keep]], starts[keep]))
+
+    def _regenerate_interesting(self):
+        hits = [r for r, _ in self._hits]
+        if not hits or not sum(len(r) for r in hits):
+            return []
+        return self.env.regenerate(np.concatenate(hits), t_global_start=np.concatenate([s for _, s in self._hits]))
 
     def _learner(self):
         """The Q-learning ego on the tensor API (config.json's stock ego option), or None when every agent is on the device."""
@@ -134,7 +171,10 @@ class BatchedSimulation:
         from . import sharding
         target = self.config.episodes if episodes is None else int(episodes)
         env = self.env
-        logging_rows = self.episode_file is not None or self.keep_rows
+        logging_rows = self.episode_file is not None or self.keep_rows or self.save_interesting > 0
+        if self.save_interesting and self.config.ego_config.agent is AgentType.Q_LEARNING:
+            raise ValueError("save_interesting regenerates episodes on the device: the Q-learning ego chooses its actions on the host")
+        self._hits = []
         if logging_rows:   # an episode lasts tens of steps at least: room for every env to finish chunk/16 times between drains
             env.set_episode_log(env.num_envs * max(1, self.chunk // 16) + 1024)
         env.reset()
@@ -162,4 +202,6 @@ class BatchedSimulation:
         self.console.info(summary.console_message())
         if self.run_file:
             self.run_file.info(summary.file_message())
+        if self.save_interesting:
+            self.interesting = self._regenerate_interesting()
         return summary

@@ -11,7 +11,8 @@ Each round is reset() followed by rollout(max_timesteps, auto_reset=False): ever
 round, so each episode is counted once and none is cut short by the end of the run (crude Monte Carlo over whole episodes,
 DESIGN §3.3).  A point therefore gets rounds * n_p episodes, the first multiple of n_p at or above --episodes.  Per point the
 results are reduced from the drained episode rows; the reference's config.json / episode.log / run.log are written under
-<log-dir>/<name>=<value>/ in experiments.py's style.
+<log-dir>/<name>=<value>/ in experiments.py's style.  --save-interesting K also writes the full trajectories of the first K
+interesting episodes of each point there, as interesting.npz (BatchedCAVEnv.regenerate, trajectories.save_episodes).
 """
 import argparse
 import dataclasses
@@ -25,6 +26,27 @@ from . import _abi, reporting
 
 PARAMETERS = {"epsilon": (_abi.CAV_AGENT_RANDOM, _abi.CAV_AGENT_RANDOM_CONSTRAINED),
               "threshold": (_abi.CAV_AGENT_PROXIMITY, _abi.CAV_AGENT_ELECTION)}
+
+
+def with_round(rows, round_index):
+    """Drained episode rows with a "round" field appended: the sweep round that played them.  An episode's rows carry no start
+    time; round r of a sweep on a fresh engine starts at t_global = r * max_timesteps (start_steps)."""
+    out = np.zeros(rows.shape, dtype=np.dtype(rows.dtype.descr + [("round", "<i4")]))
+    for field in rows.dtype.names:
+        out[field] = rows[field]
+    out["round"] = round_index
+    return out
+
+
+def start_steps(rows, max_timesteps):
+    """The t_global at the first step of each row's episode: every round is reset() + rollout(max_timesteps), so round r
+    starts at r * max_timesteps."""
+    return np.asarray(rows["round"], dtype=np.int64) * int(max_timesteps)
+
+
+def interesting_rows(rows, k):
+    """The first k rows (in drain order) of episodes a tester won (winner > 0)."""
+    return rows[rows["winner"] > 0][:int(k)]
 
 
 def point_slices(n_points, envs_per_point):
@@ -87,7 +109,8 @@ def parameter_grid(env, name, values, envs_per_point):
 def run(env, name, values, envs_per_point, episodes, env_offset=0):
     """Sweep `name` over `values` on `env`, an engine of len(values) * envs_per_point envs (and global env ids from
     env_offset).  Rounds of reset() + rollout(max_timesteps, auto_reset=False) until every point has at least `episodes`
-    episodes.  Returns (list of PointResult, list of per-point row arrays)."""
+    episodes.  Returns (list of PointResult, list of per-point row arrays); the rows carry the round that played them
+    (with_round)."""
     import torch
     n_points = len(values)
     if env.num_envs != n_points * envs_per_point:
@@ -99,7 +122,7 @@ def run(env, name, values, envs_per_point, episodes, env_offset=0):
     rounds = max(1, math.ceil(episodes / envs_per_point))
     start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     seconds, parts = 0.0, [[] for _ in range(n_points)]
-    for _ in range(rounds):
+    for round_index in range(rounds):
         start.record()
         env.reset()
         env.rollout(env.max_timesteps, auto_reset=False)
@@ -109,7 +132,7 @@ def run(env, name, values, envs_per_point, episodes, env_offset=0):
         rows, dropped = env.drain_episodes()
         if dropped or rows.size != env.num_envs:
             raise RuntimeError(f"a round drained {rows.size} episode rows ({dropped} dropped) from {env.num_envs} envs")
-        for p, chunk in enumerate(group_rows(rows, n_points, envs_per_point, env_offset)):
+        for p, chunk in enumerate(group_rows(with_round(rows, round_index), n_points, envs_per_point, env_offset)):
             parts[p].append(chunk)
     per_point = [np.concatenate(chunks) for chunks in parts]
     return [summarise(rows, name, values[p], seconds) for p, rows in enumerate(per_point)], per_point
@@ -137,6 +160,22 @@ def write_logs(config, name, results, per_point, log_root, resolution):
         run_file.info(summary.file_message())
 
 
+def save_interesting(env, name, results, per_point, log_root, k, meta=None):
+    """The first k interesting episodes of each point, regenerated on `env` (the sweep's engine, its parameters still set) with
+    the start step of their round, written to <log_root>/<name>=<value>/interesting.npz (trajectories.save_episodes).  The
+    file's meta is `meta` plus the point's parameter.  Returns the per-point lists of episodes."""
+    from . import trajectories
+    out = []
+    for result, rows in zip(results, per_point):
+        hits = interesting_rows(rows, k)
+        episodes = env.regenerate(hits, t_global_start=start_steps(hits, env.max_timesteps)) if hits.size else []
+        log_dir = f"{log_root}/{name}={result.value:g}"
+        os.makedirs(log_dir, exist_ok=True)
+        trajectories.save_episodes(f"{log_dir}/interesting.npz", episodes, dict(meta or {}, **{name: result.value}))
+        out.append(episodes)
+    return out
+
+
 def main(argv=None):
     from .config import AgentType, make_config
     parser = argparse.ArgumentParser(description="Sweep a tester parameter across the envs of one batch.")
@@ -149,7 +188,11 @@ def main(argv=None):
     parser.add_argument("--log-dir", default=None, help="write each point's config.json / episode.log / run.log under it")
     parser.add_argument("--seed", type=int, default=None, help="default: the config's seed")
     parser.add_argument("--dtype", default="float64", choices=("float64", "float32"))
+    parser.add_argument("--save-interesting", type=int, default=0, metavar="K",
+                        help="write the trajectories of the first K interesting episodes of each point to <log-dir>/<point>/interesting.npz")
     args = parser.parse_args(argv)
+    if args.save_interesting < 0 or (args.save_interesting and not args.log_dir):
+        parser.error("--save-interesting takes K >= 0 and needs --log-dir")
     name = "epsilon" if args.epsilon is not None else "threshold"
     values = [float(v) for v in (args.epsilon if name == "epsilon" else args.threshold).split(",") if v.strip()]
     with open(args.config, encoding="utf-8") as handle:
@@ -162,6 +205,9 @@ def main(argv=None):
     results, per_point = run(env, name, values, args.envs_per_point, args.episodes or config.episodes)
     if args.log_dir:
         write_logs(config, name, results, per_point, args.log_dir, env.time_resolution)
+    if args.save_interesting:
+        save_interesting(env, name, results, per_point, args.log_dir, args.save_interesting,
+                         {"config": config.to_data(), "dtype": args.dtype, "seed": (config.seed or 0) if args.seed is None else args.seed})
     env.close()
     for result in results:
         print(json.dumps(result.to_data()))

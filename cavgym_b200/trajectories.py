@@ -5,7 +5,10 @@ where the env did not step, so an episode starts at a row with timestep 1 and en
 done == 1, or one cut off at max_timesteps (done stays 0 there; the next row of the env is 0 or 1, a new episode or a
 frozen env).  complete_episodes returns the episodes that start and end inside the record, each in the per-episode layout
 of the reference's fixtures (tests/golden/*.npz), so the replay path and the oracle take them as they take those.
+save_episodes / load_episodes write and read such episodes as one .npz file in the fixtures' layout.
 """
+import json
+
 import numpy as np
 
 NEEDED = ("observation", "action", "state", "reward", "done", "winner", "tangent", "timestep")
@@ -55,3 +58,26 @@ def complete_episodes(record, t_global_start, env_offset=0, max_timesteps=None):
                 "tangent": rec["tangent"][s:u, e].copy(),
             })
     return episodes
+
+
+def save_episodes(path, episodes, meta):
+    """Episodes (dicts of arrays and numbers, as complete_episodes or BatchedCAVEnv.regenerate return them) to one .npz in the
+    layout of tests/golden: "meta" (JSON of `meta`, as uint8 bytes), "n_episodes", and "ep<i>_<field>" per episode.  A field
+    that is None is left out."""
+    arrays = {"meta": np.frombuffer(json.dumps(meta).encode(), dtype=np.uint8), "n_episodes": np.int64(len(episodes))}
+    for i, episode in enumerate(episodes):
+        for key, value in episode.items():
+            if value is not None:
+                arrays[f"ep{i}_{key}"] = np.asarray(value)
+    np.savez(path, **arrays)
+
+
+def load_episodes(path):
+    """(meta, episodes) of a file written by save_episodes (or a tests/golden fixture)."""
+    with np.load(path) as data:
+        meta = json.loads(bytes(data["meta"]).decode())
+        episodes = []
+        for i in range(int(data["n_episodes"])):
+            prefix = f"ep{i}_"
+            episodes.append({k[len(prefix):]: data[k] for k in data.files if k.startswith(prefix)})
+    return meta, episodes

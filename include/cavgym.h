@@ -286,6 +286,29 @@ int cavgym_rollout_until(CavEngine* engine, int n_steps, double level, uint64_t 
  * CAV_ESTATE also for parameters on a scenario of more than CAV_SMALL_M bodies.  Synchronises `stream`. */
 int cavgym_set_agent_params(CavEngine* engine, const double* epsilon, const void* threshold, cudaStream_t stream);
 
+/* Regenerate logged episodes: every slot e of the engine (all N) becomes episode episodes[e] of global env env_ids[e] —
+ * the (env, episode) of a CavEpisodeRow, from this engine or any other of the same scenario, seed, dtype and tau — and then
+ * steps n_steps times without auto-reset.  With on-device agents an episode's states, actions, done, winner, tangent flags
+ * and liveness are a pure function of those, of its (env, episode) key (which keys its spawn and agent draws) and of the
+ * slot's tester parameters (cavgym_set_agent_params where set, the scenario's values otherwise).  So an episode played
+ * from a reset on the engine's own streams is reproduced bit for bit, K of them side by side in one launch.  t_global
+ * only adds the time-out term (quirk 1) to the rewards of one step: it is read at the first step and advances by n_steps,
+ * so set it (cavgym_set_global_timestep) to the step at which the episode started.
+ *   env_ids   device int64[N], each in [0, 2^40)     episodes  device int32[N], each >= 0
+ *   rec       as cavgym_rollout_record's (HOST struct of device pointers), NULL allowed: row 0 is the episode's first
+ *             step, rows after it ends are frozen rows.
+ * The slot's unfinished episode, if any, is abandoned as cavgym_reset counts it; counters, the episode log and t_global
+ * then behave as for cavgym_rollout_record, and an episode row carries env_ids[e], so draining this engine's log gives
+ * back the requested rows of the episodes that reproduce.  Episodes that were not played from a reset on the engine's
+ * own streams (cavgym_fork_envs or cavgym_load_envs mid-episode, cavgym_rollout_until with a salt) are not reproduced.
+ * The keys are range-checked on the device before any state changes: synchronises `stream`.
+ * CAV_EINVAL: NULL engine, env_ids or episodes, n_steps < 0, an id or episode out of range.  CAV_ESTATE: a body with
+ * CAV_AGENT_EXTERNAL (its actions came from the caller), election testers (the active player outlives episodes, so an
+ * episode depends on the ones before it), the warp-per-environment path (more than CAV_SMALL_M bodies, or
+ * cavgym_set_dense_path(1)), a uniform or spawn override set. */
+int cavgym_regenerate_episodes(CavEngine* engine, const int64_t* env_ids, const int32_t* episodes, int n_steps,
+                               const CavRolloutRecord* rec, cudaStream_t stream);
+
 /* Replayed joint actions, n_steps transitions in one launch:
  * actions real[T][M][2][N]; trajectory outputs (each nullable) state real[T][M][4][N],
  * reward real[T][M][N], done u8[T][N], winner i32[T][N], tangent u8[T][N].
